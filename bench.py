@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """Benchmark of the sliCQT hot path (BASELINE.json metric: fwd+inv audio-seconds per second).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--batch B]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--batch B] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Workload = BASELINE.json configs[1]: the sliCQT path of a realtime-model demix of one synthetic 30 s
@@ -350,6 +350,38 @@ def bind_rank_to_cores(local_rank: int, local_world: int):
     return info
 
 
+DUMP_COEFS = 3 << 20             # complex coefficients kept by --dump-outputs (24 MiB as float32 pairs)
+DUMP_SAMPLES = 6 << 20           # waveform samples kept by --dump-outputs (24 MiB)
+
+
+def _sample(flat, n: int, seed: int):
+    """A fixed sample of a flat device tensor: up to n distinct positions (all of them if it has no more), drawn from
+    a seeded CPU generator and sorted, so that every run with the same arguments picks the same elements."""
+    N = flat.numel()
+    if N <= n:
+        return flat
+    import torch
+    idx = torch.unique(torch.randint(N, (n,), generator=torch.Generator().manual_seed(seed)))   # sorted
+    return flat[idx.to(flat.device)]
+
+
+def dump_outputs(out_dir: str, coefs, y) -> dict:
+    """Write what one step of the timed path returned: the forward coefficients (every bucket [rows, F_b, S, M_b]
+    complex64, flattened in bucket order and sampled, stored as float32 [n, 2] real / imaginary pairs) and the inverse
+    output (4 target waveforms, [targets * rows, T] float32, flattened and sampled).  Returns {name: shape}."""
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    flat_c = torch.cat([c.reshape(-1) for c in coefs])
+    out = {"forward_coefficients": torch.view_as_real(_sample(flat_c, DUMP_COEFS, 0)),
+           "inverse_waveforms": _sample(y.reshape(-1), DUMP_SAMPLES, 1)}
+    shapes = {}
+    for name, t in out.items():
+        a = t.cpu().numpy()
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+        shapes[name] = list(a.shape)
+    return shapes
+
+
 _JSON_FD = None
 
 
@@ -376,7 +408,11 @@ def main():
     _claim_stdout()
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=50)
+    ap.add_argument("--steps", type=int, default=50,
+                    help="timed steps of the headline measurement (value, ms_per_step; --mode slices and --impl "
+                         "reference too); the secondary blocks of the default line use fixed counts: e2e "
+                         "min(steps, 20) with at least 3, single_mixture and fused_step 20, slice_sharding 20, "
+                         "cpu_baseline 5")
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--batch", type=int, default=8, help="30 s mixtures per GPU per step (Separator.forward takes a batch)")
@@ -387,7 +423,14 @@ def main():
     ap.add_argument("--tracks", type=int, default=1024, help="--mode sweep: number of 3-min tracks")
     ap.add_argument("--cpu-sample-seconds", type=float, default=10.0)
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed (a fixed sample of the coefficients "
+                         "and waveforms, at most 48 MiB) as DIR/<name>.npy, to compare two builds output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "b200" or args.mode != "tracks"):
+        ap.error("--dump-outputs applies to the default workload (--impl b200 --mode tracks)")
     args.warmup = max(args.warmup, 3)
 
     rank = int(os.environ.get("RANK", "0"))
@@ -496,6 +539,8 @@ def main():
     barrier()
     launches = plan.launch_count() - launches0
     clocks = sampler.stop()
+    # the passes below reuse Cout and yout: take the timed path's outputs first
+    dumped = dump_outputs(args.dump_outputs, Cout, yout) if args.dump_outputs and rank == 0 else None
     step_ms = np.asarray([a.elapsed_time(b) for a, b in ev], dtype=np.float64)
     ms_per_step = float(step_ms.mean())
     t = torch.tensor([ms_per_step], device=dev, dtype=torch.float64)
@@ -759,7 +804,7 @@ def main():
                "ms_per_sample": dt * 1e3}
 
     if rank == 0:
-        emit(({
+        line = {
             "metric": "sliCQT fwd+inv audio-sec/sec", "value": value, "unit": "audio-s/s", "n_gpus": n_gpus,
             "steps": args.steps, "warmup": args.warmup, "ms_per_step": ms_per_step, "higher_is_better": True,
             "scaling": "weak", "vs_baseline": None, "dtype": "f32", "data": "synthetic", "config": base_cfg,
@@ -767,7 +812,10 @@ def main():
             "slice_sharding": shard,
             "gpu_launches": int(launches),
             "clocks": clocks, "max_abs_err_target0": err,
-        }))
+        }
+        if dumped is not None:
+            line["dumped_outputs"] = {"dir": args.dump_outputs, "shapes": dumped}
+        emit(line)
     if distributed:
         dist.destroy_process_group()
 
