@@ -60,7 +60,8 @@ typedef struct slicq_tables {
 /* Plan flag: the ANALYSIS entry of this plan computes the adjoint (transpose) of the SYNTHESIS of the
  * normal plan -- used for autograd through INSGT_SL (the reference gets it from torch autograd on
  * nsgt/nsigtf.py + nsgt/unslicing.py).  The slice spectrum is scaled by 2/L (1/L at DC / Nyquist) and
- * bins reaching outside [0, L/2] read zeros instead of the Hermitian mirror; the caller passes
+ * bins reaching outside [0, L/2] read zeros instead of the Hermitian mirror; for bins that reach below DC the
+ * analysis also adds the adjoint of the synthesis' mirrored-bin pass (nsgt/nsigtf.py:63-80).  The caller passes
  * tukey = 1 and win_fwd = gd * M^2. */
 #define SLICQ_PLAN_ADJOINT_OF_SYNTHESIS 1
 /* Plan flag: the SYNTHESIS entry of this plan computes the adjoint (transpose) of the ANALYSIS of the normal plan --

@@ -5,7 +5,7 @@
 // (one output per thread and stage: O(N sum p) operations, any factor, natural order in and out; twiddles from one table
 // exp(-2 pi i k / N)).  Correct for every N that fits two buffers in shared memory, not tuned: the roofline work is the
 // pretrained configuration's.  Also here: the reference's mirrored-bin pass (nsgt/nsigtf.py:63-80) for configurations
-// where a bin reaches below DC, so that its mirror image wraps into the kept half spectrum.
+// where a bin reaches below DC, so that its mirror image wraps into the kept half spectrum, and its transpose.
 #include "slicq_common.cuh"
 
 #define SLICQ_GEN_THREADS 256
@@ -129,6 +129,7 @@ __global__ void __launch_bounds__(SLICQ_GEN_THREADS, 1) slice_fft_inv_generic_ke
     __syncthreads();
     for (int i = tid; i < p.t.n_ex; i += NT) {
         const int4 q = __ldg(p.t.ex + i);
+        if (q.w) continue;                      // folded entries: below
         float2 e = __ldg(Trow + q.y);
         if (q.z >= 0) { const float2 v = __ldg(Trow + q.z); e.x += v.x; e.y += v.y; }
         A[q.x].x += e.x; A[q.x].y += e.y;
@@ -142,6 +143,16 @@ __global__ void __launch_bounds__(SLICQ_GEN_THREADS, 1) slice_fft_inv_generic_ke
         for (int f = 1 + tid; f <= p.t.pad_r; f += NT) {
             const float2 a = __ldg(P0 + N + f), b = __ldg(P1 + N + f);
             A[N - f].x += a.x + b.x; A[N - f].y -= a.y + b.y;
+        }
+        // overflow entries below DC / above Nyquist fold back conjugated, like the plane margins above: their targets
+        // coincide with those of the margins and of the direct entries, so in a pass of their own (distinct targets)
+        __syncthreads();
+        for (int i = tid; i < p.t.n_ex; i += NT) {
+            const int4 q = __ldg(p.t.ex + i);
+            if (!q.w) continue;
+            float2 e = __ldg(Trow + q.y);
+            if (q.z >= 0) { const float2 v = __ldg(Trow + q.z); e.x += v.x; e.y += v.y; }
+            A[q.x].x += e.x; A[q.x].y -= e.y;
         }
     }
     __syncthreads();
@@ -191,38 +202,82 @@ __global__ void __launch_bounds__(SLICQ_GEN_THREADS, 1) slice_fft_inv_generic_ke
 // matters only where that copy lands in the kept half [0, L/2], i.e. for a bin that reaches below DC (pos_j < M_j / 2):
 // spectrum position f = m - pos_j (m in [pos_j, M_j/2)) receives conj(t[m + 1]) * gd_mirror[m] * M_j.  In the reference's
 // rotated-slice bookkeeping this term picks up -/+ i on even / odd slices on top of the bin's sign (DESIGN.md): the entry
-// weight carries (-1)^(pos/2) M gd / L, the kernel the slice parity.  One thread per (unit, entry): t[m + 1] by a direct
-// M-term sum over the caller's coefficients, added to the plane-0 position (after bins_inv_kernel, before the slice
-// kernel, same stream: a fixed order, so the result stays deterministic).
+// weight carries (-1)^(pos/2) M gd / L, the kernel the slice parity.  One thread per (unit, position f): for every
+// mirrored bin that reaches f, in bin order, t[m + 1] by a direct M-term sum over the caller's coefficients; then ONE
+// read-modify-write of the plane-0 position (after bins_inv_kernel, before the slice kernel, same stream).  No two
+// threads touch one position and the terms are added in a fixed order, so the result is deterministic.
 __global__ void mirror_fix_kernel(const __grid_constant__ SlicqBinsParams p) {
-    const int ne = p.t.n_mir;
-    const long long total = (long long)p.n_rs * ne;
+    const int nf = p.t.mir_nf;
+    const long long total = (long long)p.n_rs * nf;
     for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
-        const int u = (int)(i / ne), e = (int)(i - (long long)u * ne);
-        const SlicqMirrorEntry me = p.t.mir[e];
-        const SlicqBucketArg& b = p.b[me.bucket];
+        const int u = (int)(i / nf), f = (int)(i - (long long)u * nf);
         const int rs = p.rs0 + u;
         const int row = rs / p.S, k = rs - row * p.S;
         const int rowx = p.x_rows ? row % p.x_rows : row;
-        const float2* c = b.ptr + rowx * b.s_row + me.f_in_bucket * b.s_bin + k * b.s_slice;
-        const float* mk = b.mptr ? b.mptr + row * b.ms_row + me.f_in_bucket * b.ms_bin + k * b.ms_slice : nullptr;
-        const float2* __restrict__ tw = p.t.tw + b.tw_off;           // exp(-2 pi i j / M)
-        float2 acc = make_float2(0.f, 0.f);
-        int idx = 0;
-        for (int n = 0; n < b.M; ++n) {
-            float2 v = c[n];
-            if (mk) { v.x *= mk[n]; v.y *= mk[n]; }
-            const float2 w = __ldg(tw + idx);
-            acc.x += v.x * w.x - v.y * w.y;
-            acc.y += v.x * w.y + v.y * w.x;
-            idx += me.m_src; if (idx >= b.M) idx -= b.M;
-        }
-        // conj(t) * weight * (-i on even, +i on odd global slices)
         const bool odd = ((p.k0 + k) & 1) != 0;
-        const float2 ct = make_float2(acc.x * me.weight, -acc.y * me.weight);
-        const float2 val = odd ? make_float2(-ct.y, ct.x) : make_float2(ct.y, -ct.x);
-        float2* dst = p.spec + (long long)u * p.spec_stride + me.t_off;
-        dst->x += val.x; dst->y += val.y;
+        float2* dst = p.spec + (long long)u * p.spec_stride + p.t.pl_off + f;
+        float2 sum = *dst;
+        for (int bi = 0; bi < p.t.n_mir_bins; ++bi) {
+            const SlicqMirrorBin mb = p.t.mir_bins[bi];
+            if (f >= mb.count) continue;
+            const SlicqMirrorEntry me = p.t.mir[mb.first + f];
+            const SlicqBucketArg& b = p.b[mb.bucket];
+            const float2* c = b.ptr + rowx * b.s_row + mb.f_in_bucket * b.s_bin + k * b.s_slice;
+            const float* mk = b.mptr ? b.mptr + row * b.ms_row + mb.f_in_bucket * b.ms_bin + k * b.ms_slice : nullptr;
+            const float2* __restrict__ tw = p.t.tw + b.tw_off;           // exp(-2 pi i j / M)
+            float2 acc = make_float2(0.f, 0.f);
+            int idx = 0;
+            for (int n = 0; n < b.M; ++n) {
+                float2 v = c[n];
+                if (mk) { v.x *= mk[n]; v.y *= mk[n]; }
+                const float2 w = __ldg(tw + idx);
+                acc.x += v.x * w.x - v.y * w.y;
+                acc.y += v.x * w.y + v.y * w.x;
+                idx += me.m_src; if (idx >= b.M) idx -= b.M;
+            }
+            // conj(t) * weight * (-i on even, +i on odd global slices)
+            const float2 ct = make_float2(acc.x * me.weight, -acc.y * me.weight);
+            const float2 val = odd ? make_float2(-ct.y, ct.x) : make_float2(ct.y, -ct.x);
+            sum.x += val.x; sum.y += val.y;
+        }
+        *dst = sum;
+    }
+}
+
+// Transpose of mirror_fix_kernel under <a, b> = Re(conj(a) b), for the analysis entry of a SLICQ_PLAN_ADJOINT_OF_SYNTHESIS
+// plan.  The forward term adds s i w conj(sum_n c[n] e^{-2 pi i n q / M}) at position f (q = m_src, w the entry weight,
+// s = -1 / +1 on even / odd global slices); its transpose is
+//     c[n] += s i (L w) conj(H[f]) e^{+2 pi i n q / M},
+// H the adjoint plan's padded half spectrum (2/L, 1/L at DC, folded in; L w undoes the 1/L the weight carries for the
+// slice IFFT).  Runs after bins_fwd_kernel on the same stream.  One thread per (unit, mirrored bin, n) sums the bin's
+// entries in order and updates c[n] once: no atomics, deterministic.
+__global__ void mirror_adj_kernel(const __grid_constant__ SlicqBinsParams p) {
+    const int nc = p.t.mir_nc;
+    const long long total = (long long)p.n_rs * nc;
+    const float Lf = (float)p.t.L;
+    for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
+        const int u = (int)(i / nc);
+        int n = (int)(i - (long long)u * nc), bi = 0;
+        while (n >= p.b[p.t.mir_bins[bi].bucket].M) { n -= p.b[p.t.mir_bins[bi].bucket].M; ++bi; }
+        const SlicqMirrorBin mb = p.t.mir_bins[bi];
+        const SlicqBucketArg& b = p.b[mb.bucket];
+        const int rs = p.rs0 + u;
+        const int row = rs / p.S, k = rs - row * p.S;
+        const float2* __restrict__ H = p.spec + (long long)u * p.spec_stride + p.t.pad_l;
+        const float2* __restrict__ tw = p.t.tw + b.tw_off;           // exp(-2 pi i j / M)
+        float2 acc = make_float2(0.f, 0.f);                          // sum_f (L w) conj(H[f] e^{-2 pi i n q / M})
+        for (int f = 0; f < mb.count; ++f) {
+            const SlicqMirrorEntry me = p.t.mir[mb.first + f];
+            const float2 hw = cmul(H[f], __ldg(tw + (n * me.m_src) % b.M));
+            const float a = Lf * me.weight;
+            acc.x += a * hw.x; acc.y -= a * hw.y;
+        }
+        const bool odd = ((p.k0 + k) & 1) != 0;                       // times +i on odd, -i on even global slices
+        const float2 v = odd ? make_float2(-acc.y, acc.x) : make_float2(acc.y, -acc.x);
+        float2* c = b.ptr + row * b.s_row + mb.f_in_bucket * b.s_bin + k * b.s_slice + n;
+        float2 cv = *c;
+        cv.x += v.x; cv.y += v.y;
+        *c = cv;
     }
 }
 
@@ -270,8 +325,16 @@ extern "C" int slicq_launch_slice_inv_generic(const SlicqSliceParams* p, cudaStr
 
 extern "C" int slicq_launch_mirror_fix(const SlicqBinsParams* p, cudaStream_t s) {
     if (p->t.n_mir <= 0 || p->n_rs <= 0) return 0;
-    const long long total = (long long)p->n_rs * p->t.n_mir;
+    const long long total = (long long)p->n_rs * p->t.mir_nf;
     const int blocks = (int)((total + 127) / 128 > 4096 ? 4096 : (total + 127) / 128);
     SLICQ_LAUNCH(mirror_fix_kernel, dim3(blocks), dim3(128), 0, s, *p);
+    return (int)cudaGetLastError();
+}
+
+extern "C" int slicq_launch_mirror_adj(const SlicqBinsParams* p, cudaStream_t s) {
+    if (p->t.n_mir <= 0 || p->n_rs <= 0) return 0;
+    const long long total = (long long)p->n_rs * p->t.mir_nc;
+    const int blocks = (int)((total + 127) / 128 > 4096 ? 4096 : (total + 127) / 128);
+    SLICQ_LAUNCH(mirror_adj_kernel, dim3(blocks), dim3(128), 0, s, *p);
     return (int)cudaGetLastError();
 }

@@ -1,7 +1,9 @@
 // C-ABI of libslicq (include/slicq.h): plan construction and the chunked launch sequences.
 //
-// forward  : per chunk of (row,slice) units   slice_fft_fwd_kernel -> bins_fwd_kernel
-// inverse  : per chunk                         bins_inv_kernel -> slice_fft_inv_kernel (even slices, then odd slices)
+// forward  : per chunk of (row,slice) units   slice_fft_fwd_kernel -> bins_fwd_kernel [-> mirror_adj_kernel]
+// inverse  : per chunk                         bins_inv_kernel [-> mirror_fix_kernel] -> slice_fft_inv_kernel (even slices,
+//                                              then odd slices)
+// (the bracketed kernels only for bins that reach below DC; mirror_adj_kernel only in the adjoint-of-synthesis plan)
 // A chunk's intermediate spectra (analysis: padded half spectra H; synthesis: the two bin planes T) live in the
 // caller-provided scratch buffer; SLICQ_CHUNK_MB bounds the chunk (default: one chunk per call).
 #include "slicq_common.cuh"
@@ -57,8 +59,11 @@ extern "C" int slicq_launch_slice_inv(const SlicqSliceParams* p, cudaStream_t s)
 extern "C" int slicq_slice_smem_bytes(int L);
 extern "C" int slicq_bins_threads(void);
 extern "C" int slicq_launch_mirror_fix(const SlicqBinsParams* p, cudaStream_t s);
+extern "C" int slicq_launch_mirror_adj(const SlicqBinsParams* p, cudaStream_t s);
 
 namespace {
+
+const int kTunedSliceLen = 18060;      // slice length of the tuned prime-factor slice kernels (k_slice.cu, 2 * Pfa9030::N)
 
 thread_local std::string g_err;
 std::atomic<long long> g_launches{0};
@@ -345,17 +350,36 @@ extern "C" int slicq_plan_create(const slicq_tables* t, slicq_plan** out) {
         for (int j = b.first_bin; j < b.first_bin + b.n_bins; ++j)
             if ((b.kind == 2 && ov[j] > b.A) || (b.kind == 3 && ov[j] > b.B)) { delete p; return fail(SLICQ_E_UNSUPPORTED, "overlap between bins of one plane exceeds the first transform pass"); }
     p->t_stride = (2LL * pl_len + n_ovf + 1) & ~1LL;
+    // overflow entries, one per target position.  The synthesis drops the parts outside [0, N2]; the adjoint of the analysis
+    // folds them back conjugated (the analysis reads the Hermitian mirror there), as separate entries after the direct ones:
+    // their targets may coincide with direct targets, so the slice kernel adds them in a later pass
     std::vector<int4> ex;
     {
-        std::vector<int> e0(N2 + 1, -1), e1(N2 + 1, -1);
+        const bool fold = (t->flags & SLICQ_PLAN_ADJOINT_OF_ANALYSIS) != 0;
+        std::vector<int> e0(N2 + 1, -1), e1(N2 + 1, -1), c0(N2 + 1, -1), c1(N2 + 1, -1);
         for (int j = 0; j < J; ++j)
             for (int m = 0; m < ov[j]; ++m) {
-                const int f = p->bin_pos[j] - p->bin_M[j] / 2 + m;
-                if (f < 0 || f > N2) continue;
-                if (e0[f] < 0) e0[f] = ovoff[j] + m; else e1[f] = ovoff[j] + m;
+                int f = p->bin_pos[j] - p->bin_M[j] / 2 + m;
+                const bool out = f < 0 || f > N2;
+                if (out && !fold) continue;
+                if (f < 0) f = -f;
+                if (f > N2) f = 2 * N2 - f;
+                std::vector<int>& a = out ? c0 : e0;
+                std::vector<int>& b = out ? c1 : e1;
+                if (a[f] < 0) a[f] = ovoff[j] + m;
+                else if (b[f] < 0) b[f] = ovoff[j] + m;
+                else { delete p; return fail(SLICQ_E_UNSUPPORTED, "more than two overflow entries at one spectrum position"); }
             }
         for (int f = 0; f <= N2; ++f)
             if (e0[f] >= 0) ex.push_back(int4{f, e0[f], e1[f], 0});
+        for (int f = 0; f <= N2; ++f)
+            if (c0[f] >= 0) ex.push_back(int4{f, c0[f], c1[f], 1});
+        // the tuned slice kernels (k_slice.cu) have no folded pass
+        if (L == kTunedSliceLen && ex.size() > 0 && ex.back().w) {
+            delete p;
+            return fail(SLICQ_E_UNSUPPORTED, "adjoint of the analysis: overflow below DC / above Nyquist is not implemented in "
+                                             "the tuned slice kernels (slice length 18060)");
+        }
     }
     const int n_ex = (int)ex.size();
     if (ex.empty()) ex.push_back(int4{0, 0, -1, 0});
@@ -391,16 +415,21 @@ extern "C" int slicq_plan_create(const slicq_tables* t, slicq_plan** out) {
     }
     if (gaps.empty()) gaps.push_back(int2{0, 0});
     // mirrored-bin entries (see mirror_fix_kernel): bin j >= 1 with pos_j < M_j / 2; reference-order index m in [pos_j, M_j/2)
+    // lands at spectrum position f = m - pos_j (< pad_l <= N2 / 2)
     std::vector<SlicqMirrorEntry> mir;
+    std::vector<SlicqMirrorBin> mir_bins;
+    int mir_nf = 0, mir_nc = 0;
     for (size_t bi = 0; bi < p->buckets.size(); ++bi) {
         const Bucket& b = p->buckets[bi];
         for (int j = std::max(1, b.first_bin); j < std::min(J - 1, b.first_bin + b.n_bins); ++j) {
             const int M = b.M, pos = p->bin_pos[j];
+            if (pos >= M / 2) continue;
+            mir_bins.push_back(SlicqMirrorBin{(int)bi, j - b.first_bin, (int)mir.size(), M / 2 - pos});
+            mir_nf = std::max(mir_nf, M / 2 - pos);
+            mir_nc += M;
             for (int m = pos; m < M / 2; ++m) {
-                const int f = m - pos;
-                if (f > N2) continue;
                 SlicqMirrorEntry e;
-                e.bucket = (int)bi; e.f_in_bucket = j - b.first_bin; e.m_src = m + 1; e.t_off = pl_off + f;
+                e.m_src = m + 1;
                 const double gdm = (double)t->win_inv[p->bin_coff[j] + (M - m) % M];      // dual window of the mirrored bin at m
                 const double sgn = (((pos / 2) + m) % 2) ? -1.0 : 1.0;                     // (-1)^(pos/2) (-1)^m
                 e.weight = (float)(sgn * gdm * (double)M / (double)L);
@@ -408,9 +437,12 @@ extern "C" int slicq_plan_create(const slicq_tables* t, slicq_plan** out) {
             }
         }
     }
-    // (the adjoint-of-analysis plan has no such pass: the analysis reads the exact Hermitian mirror)
+    // (the adjoint-of-analysis plan has no such pass: the analysis reads the exact Hermitian mirror; the adjoint-of-synthesis
+    // plan runs the pass's transpose, mirror_adj_kernel, after its analysis bins)
     const int n_mir = (getenv("SLICQ_NO_MIRROR") || (t->flags & SLICQ_PLAN_ADJOINT_OF_ANALYSIS)) ? 0 : (int)mir.size();   // SLICQ_NO_MIRROR: verification aid (shows what the pass contributes)
-    if (mir.empty()) mir.push_back(SlicqMirrorEntry{0, 0, 0, 0, 0.f});
+    if (mir.empty()) mir.push_back(SlicqMirrorEntry{0, 0.f});
+    const int n_mir_bins = (int)mir_bins.size();
+    if (mir_bins.empty()) mir_bins.push_back(SlicqMirrorBin{0, 0, 0, 0});
     // generic slice kernels: prime factors of N2 (largest first) and the table exp(-2 pi i k / N2)
     std::vector<int> fac;
     { int n = N2; for (int d = 2; d * d <= n; ++d) while (n % d == 0) { fac.push_back(d); n /= d; } if (n > 1) fac.push_back(n); }
@@ -448,9 +480,11 @@ extern "C" int slicq_plan_create(const slicq_tables* t, slicq_plan** out) {
     rc |= upload(ex, &d.ex, p->owned);
     rc |= upload(gaps, &d.gaps, p->owned);
     rc |= upload(mir, &d.mir, p->owned);
+    rc |= upload(mir_bins, &d.mir_bins, p->owned);
     rc |= upload(wN, &d.wN, p->owned);
     rc |= upload(wP, &d.wP, p->owned);
     d.n_mir = n_mir; d.n_fac = (int)fac.size();
+    d.n_mir_bins = n_mir_bins; d.mir_nf = mir_nf; d.mir_nc = mir_nc;
     for (size_t i = 0; i < fac.size(); ++i) d.fac[i] = fac[i];
     d.n_ex = n_ex; d.pl_off = pl_off; d.pl_len = pl_len; d.t_stride = (int)p->t_stride;
     if (rc) {
@@ -671,6 +705,7 @@ int forward_one(const slicq_plan* p, const float* x, int64_t n_rows, int64_t x_r
     sp.spec = H; sp.spec_stride = p->spec_stride_fwd; sp.S = (int)n_slices;
     SlicqBinsParams* bp = new SlicqBinsParams();
     bp->t = p->dev; bp->spec = H; bp->spec_stride = p->spec_stride_fwd; bp->S = (int)n_slices;
+    bp->k0 = (int)k0;
     int rc = 0;
     for (long long u0 = 0; u0 < units && rc == 0; u0 += cu) {
         const int n = (int)((units - u0 < cu) ? (units - u0) : cu);
@@ -682,6 +717,11 @@ int forward_one(const slicq_plan* p, const float* x, int64_t n_rows, int64_t x_r
         const int jobs = fill_bins_params(p, buckets, *bp, n, nullptr, norms);
         { ProfScope ps(K_BINS_FWD, s); rc = slicq_launch_bins(bp, jobs, p->bins_smem, 0, s); }
         ++g_launches;
+        if (rc) break;
+        if ((p->dev.adjoint & 1) && p->dev.n_mir > 0) {      // transpose of the mirrored-bin pass, reads this chunk's H
+            rc = slicq_launch_mirror_adj(bp, s);
+            ++g_launches;
+        }
     }
     delete bp;
     if (rc) {

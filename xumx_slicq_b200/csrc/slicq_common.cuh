@@ -201,8 +201,10 @@ SLICQ_DEVFN float2 cmul_conj(float2 a, float2 b) {  // a * conj(b)
 SLICQ_DEVFN float2 cconj(float2 a) { return make_float2(a.x, -a.y); }
 
 // ---------------------------------------------------------------------------------------
-// mirrored-bin pass of the reference (nsigtf.py:63-80) for a bin that reaches below DC: one entry per spectrum position
-struct SlicqMirrorEntry { int bucket, f_in_bucket, m_src, t_off; float weight; };
+// mirrored-bin pass of the reference (nsigtf.py:63-80) for a bin that reaches below DC: one entry per spectrum position.
+// The entries of one mirrored bin are consecutive, entry first + f for spectrum position f = 0 .. count - 1.
+struct SlicqMirrorEntry { int m_src; float weight; };
+struct SlicqMirrorBin { int bucket, f_in_bucket, first, count; };
 
 // device-side tables owned by the plan (all in global memory, < 1 MB, L2 resident)
 struct SlicqDeviceTables {
@@ -237,7 +239,8 @@ struct SlicqDeviceTables {
     const int* bin_toff;          // [J] offset in the row of coefficient m' = 0 of bin j
     const int* bin_ov;            // [J] leading coefficients of bin j that go to the overflow area (even, usually 0)
     const int* bin_ovoff;         // [J] offset in the row of the overflow slot of m' = 0
-    const int4* ex;               // [n_ex] {f, off0, off1 or -1, 0}: position f also receives T[off0] (+ T[off1])
+    const int4* ex;               // [n_ex] {f, off0, off1 or -1, fold}: position f also receives T[off0] (+ T[off1]),
+                                  // conjugated if fold (adjoint of the analysis: overflow below DC / above Nyquist)
     int n_ex;
     const int2* gaps;             // {offset in the row, count}: zero-filled per unit by the job of the owning bucket
     // generic slice kernels (k_slice_generic.cu): prime factors of N2 and exp(-2 pi i k / N2)
@@ -246,7 +249,11 @@ struct SlicqDeviceTables {
     const float2* wN;
     const double2* wP;            // exp(-2 pi i k / fac[0]) in double when the largest factor is > 32 (direct sums of many terms)
     const SlicqMirrorEntry* mir;  // [n_mir]
-    int n_mir;
+    int n_mir;                    // 0: no mirrored-bin pass
+    const SlicqMirrorBin* mir_bins;   // [n_mir_bins] in bin order
+    int n_mir_bins;
+    int mir_nf;                   // spectrum positions 0 .. mir_nf - 1 receive mirrored terms (largest count)
+    int mir_nc;                   // coefficients of all mirrored bins (sum of their M)
 };
 
 // one bucket as a kernel sees it for one call (pointer + strides of the caller's tensor)

@@ -404,12 +404,9 @@ class NSGT_sliced(torch.nn.Module):
         """g [N, length] (gradient w.r.t. the synthesis output) -> per bucket [N, F_b, S, M_b] complex:
         the transpose of ``backward_rows`` with respect to the real inner product
         <y, g> = sum y*g, <c, d> = sum Re(c) Re(d) + Im(c) Im(d).  Runs on the analysis kernels
-        with a second plan (no slicing window, dual windows, zero instead of mirrored margins)."""
+        with a second plan (no slicing window, dual windows, zero instead of mirrored margins, and the transpose of the
+        mirrored-bin pass for bins that reach below DC)."""
         _BACKEND.check(g)
-        t = self.tables
-        if any(int(t.bin_pos[j]) < int(t.bin_M[j]) // 2 for j in range(1, t.n_bins - 1)):
-            raise NotImplementedError("gradients through the synthesis are not implemented for configurations whose "
-                                      "bins reach below DC (the reference's mirrored-bin pass has no adjoint kernel here)")
         if self._adj_tables is None:
             self._adj_tables = _AdjointTables(self.tables)
         if g.dtype != torch.float32:
