@@ -149,6 +149,21 @@ int slicq_inverse_masked(const slicq_plan* plan, const slicq_bucket_view* mix, c
                          int64_t y_row_stride, int64_t length, int64_t t0, float* halo_out, void* scratch,
                          size_t scratch_bytes, void* stream);
 
+/* Gradient of slicq_inverse_masked with respect to its masks, for autograd through the fused synthesis.  Only valid on
+ * a plan created with SLICQ_PLAN_ADJOINT_OF_SYNTHESIS (SLICQ_E_INVALID otherwise).  g: n_targets * n_rows rows of
+ * float32 (row r at g + r*g_row_stride, n_samples valid samples from global sample t0), the gradient with respect to
+ * slicq_inverse_masked's output in the same row order; mix: the n_rows MIXTURE rows that call read (read only).
+ * grad_masks[b] (fp32, logical shape [n_targets * n_rows][F_b][S][M_b], strides in floats, M contiguous) receives
+ *     grad[t * n_rows + r] = Re(conj(mix[r]) * (S^T g)[t * n_rows + r]),
+ * S^T g the adjoint of the synthesis that this plan's analysis computes.  The product with the mixture is taken in the
+ * epilogue of the per-bin transforms (and of the mirrored-bin adjoint for bins that reach below DC), so S^T g is never
+ * written: 8 bytes read and 4 written per coefficient and target.  Scratch: slicq_scratch_bytes(plan,
+ * n_targets * n_rows, n_slices, 0). */
+int slicq_forward_mask_grad(const slicq_plan* plan, const float* g, int64_t n_targets, int64_t n_rows,
+                            int64_t g_row_stride, int64_t n_samples, int64_t t0, int64_t k0, int64_t n_slices,
+                            const slicq_bucket_view* mix, const slicq_bucket_view* grad_masks,
+                            void* scratch, size_t scratch_bytes, void* stream);
+
 /* number of kernel launches issued by this library since load (bench bookkeeping) */
 int64_t slicq_launch_count(void);
 

@@ -23,7 +23,8 @@ SLICQ_E_SCRATCH = -4
 EXPORTS = (
     "slicq_abi_version", "slicq_build_kind", "slicq_last_error", "slicq_plan_create", "slicq_plan_destroy",
     "slicq_plan_n_buckets", "slicq_plan_bucket_info", "slicq_plan_num_slices",
-    "slicq_scratch_bytes", "slicq_forward", "slicq_forward_packed", "slicq_forward_norm", "slicq_forward_packed_norm", "slicq_inverse", "slicq_inverse_masked", "slicq_launch_count",
+    "slicq_scratch_bytes", "slicq_forward", "slicq_forward_packed", "slicq_forward_norm", "slicq_forward_packed_norm", "slicq_inverse", "slicq_inverse_masked", "slicq_forward_mask_grad",
+    "slicq_launch_count",
     "slicq_profile_enable", "slicq_profile_read",
 )
 KERNEL_NAMES = ("slice_fft_fwd", "bins_fwd", "bins_inv", "slice_fft_inv")
@@ -90,6 +91,10 @@ def _declare(lib: C.CDLL) -> C.CDLL:
                                          C.c_int64, C.c_int64, C.c_void_p, C.c_int64, C.c_int64, C.c_int64, C.c_void_p,
                                          C.c_void_p, C.c_size_t, C.c_void_p]
     lib.slicq_inverse_masked.restype = C.c_int
+    lib.slicq_forward_mask_grad.argtypes = [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_int64, C.c_int64, C.c_int64,
+                                            C.c_int64, C.c_int64, C.POINTER(BucketViewC), C.POINTER(BucketViewC),
+                                            C.c_void_p, C.c_size_t, C.c_void_p]
+    lib.slicq_forward_mask_grad.restype = C.c_int
     lib.slicq_launch_count.restype = C.c_int64
     lib.slicq_profile_enable.argtypes = [C.c_int]
     lib.slicq_profile_enable.restype = C.c_int
@@ -246,6 +251,13 @@ class Plan:
             self.handle, self._views(mix_views), self._views(mask_views), n_targets, n_rows, n_slices, k0,
             C.c_void_p(y_ptr), y_row_stride, length, t0, C.c_void_p(halo_ptr) if halo_ptr else None,
             C.c_void_p(scratch_ptr), scratch_bytes, C.c_void_p(stream)))
+
+    def forward_mask_grad(self, g_ptr: int, n_targets: int, n_rows: int, g_row_stride: int, n_samples: int, t0: int,
+                          k0: int, n_slices: int, mix_views: Sequence[tuple], grad_views: Sequence[tuple],
+                          scratch_ptr: int, scratch_bytes: int, stream: int):
+        _check(self.lib, self.lib.slicq_forward_mask_grad(
+            self.handle, C.c_void_p(g_ptr), n_targets, n_rows, g_row_stride, n_samples, t0, k0, n_slices,
+            self._views(mix_views), self._views(grad_views), C.c_void_p(scratch_ptr), scratch_bytes, C.c_void_p(stream)))
 
     def launch_count(self) -> int:
         return int(self.lib.slicq_launch_count())

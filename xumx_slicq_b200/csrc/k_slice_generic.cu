@@ -250,7 +250,9 @@ __global__ void mirror_fix_kernel(const __grid_constant__ SlicqBinsParams p) {
 //     c[n] += s i (L w) conj(H[f]) e^{+2 pi i n q / M},
 // H the adjoint plan's padded half spectrum (2/L, 1/L at DC, folded in; L w undoes the 1/L the weight carries for the
 // slice IFFT).  Runs after bins_fwd_kernel on the same stream.  One thread per (unit, mirrored bin, n) sums the bin's
-// entries in order and updates c[n] once: no atomics, deterministic.
+// entries in order and updates c[n] once: no atomics, deterministic.  In the mask-gradient mode (p.mask_grad) the bins
+// kernel has stored Re(conj(X) c) instead of c, X the mixture; the same term then goes to that gradient:
+//     grad[n] += Re(conj(X[n]) v),  X read at mixture row row % x_rows.
 __global__ void mirror_adj_kernel(const __grid_constant__ SlicqBinsParams p) {
     const int nc = p.t.mir_nc;
     const long long total = (long long)p.n_rs * nc;
@@ -274,6 +276,12 @@ __global__ void mirror_adj_kernel(const __grid_constant__ SlicqBinsParams p) {
         }
         const bool odd = ((p.k0 + k) & 1) != 0;                       // times +i on odd, -i on even global slices
         const float2 v = odd ? make_float2(-acc.y, acc.x) : make_float2(acc.y, -acc.x);
+        if (p.mask_grad) {
+            const float2 x = b.ptr[(p.x_rows ? row % p.x_rows : row) * b.s_row + mb.f_in_bucket * b.s_bin + k * b.s_slice + n];
+            float* gm = b.nptr + row * b.ms_row + mb.f_in_bucket * b.ms_bin + k * b.ms_slice + n;
+            *gm += mask_grad_of(x, v);
+            continue;
+        }
         float2* c = b.ptr + row * b.s_row + mb.f_in_bucket * b.s_bin + k * b.s_slice + n;
         float2 cv = *c;
         cv.x += v.x; cv.y += v.y;

@@ -1,6 +1,7 @@
 // C-ABI of libslicq (include/slicq.h): plan construction and the chunked launch sequences.
 //
 // forward  : per chunk of (row,slice) units   slice_fft_fwd_kernel -> bins_fwd_kernel [-> mirror_adj_kernel]
+//            (slicq_forward_mask_grad: the same sequence, bins_fwd_kernel / mirror_adj_kernel in their mask-gradient mode)
 // inverse  : per chunk                         bins_inv_kernel [-> mirror_fix_kernel] -> slice_fft_inv_kernel (even slices,
 //                                              then odd slices)
 // (the bracketed kernels only for bins that reach below DC; mirror_adj_kernel only in the adjoint-of-synthesis plan)
@@ -623,7 +624,8 @@ int fill_bins_params(const slicq_plan* p, const slicq_bucket_view* views, SlicqB
 namespace {
 int forward_one(const slicq_plan* p, const float* x, int64_t n_rows, int64_t x_row_stride,
                 int64_t n_samples, int64_t t0, int64_t k0, int64_t n_slices,
-                const slicq_bucket_view* buckets, const slicq_bucket_view* norms, void* scratch, cudaStream_t s);
+                const slicq_bucket_view* buckets, const slicq_bucket_view* norms, int64_t mix_rows, void* scratch,
+                cudaStream_t s);
 int inverse_one(const slicq_plan* p, const slicq_bucket_view* buckets, const slicq_bucket_view* masks, int64_t x_rows,
                 int64_t n_rows, int64_t n_slices, int64_t k0, float* y, int64_t y_row_stride, int64_t length,
                 int64_t t0, float* halo_out, void* scratch, cudaStream_t s);
@@ -650,10 +652,12 @@ int run_split(const slicq_plan* p, int64_t n_rows, int64_t n_slices, int inverse
 }  // namespace
 
 namespace {
+// mix_rows == 0: analysis of x into `buckets` (and |c| into `norms` when given).  mix_rows > 0: mask-gradient analysis,
+// `buckets` hold the mixture (mix_rows rows, read only) and `norms` receive the mask gradient of the n_rows output rows.
 int forward_impl(const slicq_plan* p, const float* x, int64_t n_rows, int64_t x_row_stride,
                  int64_t n_samples, int64_t t0, int64_t k0, int64_t n_slices,
-                 const slicq_bucket_view* buckets, const slicq_bucket_view* norms, void* scratch, size_t scratch_bytes,
-                 void* stream) {
+                 const slicq_bucket_view* buckets, const slicq_bucket_view* norms, int64_t mix_rows, void* scratch,
+                 size_t scratch_bytes, void* stream) {
     if (!p || !x || !buckets) return fail(SLICQ_E_INVALID, "null argument");
     if (n_rows <= 0 || n_slices <= 0 || n_samples < 0) return fail(SLICQ_E_INVALID, "bad shape");
     if (n_rows * n_slices > 0x7fffffffLL) return fail(SLICQ_E_INVALID, "too many (row,slice) units");
@@ -663,26 +667,34 @@ int forward_impl(const slicq_plan* p, const float* x, int64_t n_rows, int64_t x_
     for (size_t i = 0; i < p->buckets.size(); ++i)
         if (!buckets[i].ptr || (norms && !norms[i].ptr)) return fail(SLICQ_E_INVALID, "null bucket pointer");
     cudaStream_t s0 = reinterpret_cast<cudaStream_t>(stream);
-    if (use_split(p, n_rows, n_slices)) {
+    // mask gradient: output row r reads mixture row r % mix_rows, so a row group must start on a multiple of mix_rows
+    bool split = use_split(p, n_rows, n_slices);
+    if (split && mix_rows) {
+        const int ways = split_ways(p, n_rows);
+        for (int h = 1; h < ways; ++h) split = split && (part_row0(n_rows, ways, h) % mix_rows == 0);
+    }
+    if (split) {
         return run_split(p, n_rows, n_slices, 0, scratch, s0, [&](int64_t r0, int64_t rows, void* scr, cudaStream_t st) {
             std::vector<slicq_bucket_view> v(buckets, buckets + p->buckets.size()), nv;
-            for (auto& b : v) b.ptr = reinterpret_cast<float2*>(b.ptr) + r0 * b.s_row;
+            if (!mix_rows)      // the mixture is shared by all row groups
+                for (auto& b : v) b.ptr = reinterpret_cast<float2*>(b.ptr) + r0 * b.s_row;
             if (norms) {
                 nv.assign(norms, norms + p->buckets.size());
                 for (auto& b : nv) b.ptr = reinterpret_cast<float*>(b.ptr) + r0 * b.s_row;
             }
             return forward_one(p, x + r0 * x_row_stride, rows, x_row_stride, n_samples, t0, k0, n_slices, v.data(),
-                               norms ? nv.data() : nullptr, scr, st);
+                               norms ? nv.data() : nullptr, mix_rows, scr, st);
         });
     }
-    return forward_one(p, x, n_rows, x_row_stride, n_samples, t0, k0, n_slices, buckets, norms, scratch, s0);
+    return forward_one(p, x, n_rows, x_row_stride, n_samples, t0, k0, n_slices, buckets, norms, mix_rows, scratch, s0);
 }
 }  // namespace
 
 extern "C" int slicq_forward(const slicq_plan* p, const float* x, int64_t n_rows, int64_t x_row_stride,
                              int64_t n_samples, int64_t t0, int64_t k0, int64_t n_slices,
                              const slicq_bucket_view* buckets, void* scratch, size_t scratch_bytes, void* stream) {
-    return forward_impl(p, x, n_rows, x_row_stride, n_samples, t0, k0, n_slices, buckets, nullptr, scratch, scratch_bytes, stream);
+    return forward_impl(p, x, n_rows, x_row_stride, n_samples, t0, k0, n_slices, buckets, nullptr, 0, scratch, scratch_bytes,
+                        stream);
 }
 
 extern "C" int slicq_forward_norm(const slicq_plan* p, const float* x, int64_t n_rows, int64_t x_row_stride,
@@ -690,13 +702,26 @@ extern "C" int slicq_forward_norm(const slicq_plan* p, const float* x, int64_t n
                                   const slicq_bucket_view* buckets, const slicq_bucket_view* norms, void* scratch,
                                   size_t scratch_bytes, void* stream) {
     if (!norms) return fail(SLICQ_E_INVALID, "norms missing");
-    return forward_impl(p, x, n_rows, x_row_stride, n_samples, t0, k0, n_slices, buckets, norms, scratch, scratch_bytes, stream);
+    return forward_impl(p, x, n_rows, x_row_stride, n_samples, t0, k0, n_slices, buckets, norms, 0, scratch, scratch_bytes,
+                        stream);
+}
+
+extern "C" int slicq_forward_mask_grad(const slicq_plan* p, const float* g, int64_t n_targets, int64_t n_rows,
+                                       int64_t g_row_stride, int64_t n_samples, int64_t t0, int64_t k0, int64_t n_slices,
+                                       const slicq_bucket_view* mix, const slicq_bucket_view* grad_masks,
+                                       void* scratch, size_t scratch_bytes, void* stream) {
+    if (!p || !grad_masks || n_targets <= 0 || n_rows <= 0) return fail(SLICQ_E_INVALID, "null argument or bad shape");
+    if (!(p->dev.adjoint & SLICQ_PLAN_ADJOINT_OF_SYNTHESIS))
+        return fail(SLICQ_E_INVALID, "the mask gradient needs a plan created with SLICQ_PLAN_ADJOINT_OF_SYNTHESIS");
+    return forward_impl(p, g, n_targets * n_rows, g_row_stride, n_samples, t0, k0, n_slices, mix, grad_masks, n_rows,
+                        scratch, scratch_bytes, stream);
 }
 
 namespace {
 int forward_one(const slicq_plan* p, const float* x, int64_t n_rows, int64_t x_row_stride,
                 int64_t n_samples, int64_t t0, int64_t k0, int64_t n_slices,
-                const slicq_bucket_view* buckets, const slicq_bucket_view* norms, void* scratch, cudaStream_t s) {
+                const slicq_bucket_view* buckets, const slicq_bucket_view* norms, int64_t mix_rows, void* scratch,
+                cudaStream_t s) {
     const long long units = n_rows * n_slices, cu = chunk_units(p, 0);
     float2* H = reinterpret_cast<float2*>((reinterpret_cast<uintptr_t>(scratch) + 255) & ~(uintptr_t)255);
     SlicqSliceParams sp;
@@ -706,6 +731,7 @@ int forward_one(const slicq_plan* p, const float* x, int64_t n_rows, int64_t x_r
     SlicqBinsParams* bp = new SlicqBinsParams();
     bp->t = p->dev; bp->spec = H; bp->spec_stride = p->spec_stride_fwd; bp->S = (int)n_slices;
     bp->k0 = (int)k0;
+    bp->x_rows = (int)mix_rows; bp->mask_grad = mix_rows > 0;
     int rc = 0;
     for (long long u0 = 0; u0 < units && rc == 0; u0 += cu) {
         const int n = (int)((units - u0 < cu) ? (units - u0) : cu);

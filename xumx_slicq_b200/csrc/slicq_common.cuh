@@ -199,6 +199,10 @@ SLICQ_DEVFN float2 cmul_conj(float2 a, float2 b) {  // a * conj(b)
     return make_float2(fmaf(a.x, b.x, a.y * b.y), fmaf(a.y, b.x, -a.x * b.y));
 }
 SLICQ_DEVFN float2 cconj(float2 a) { return make_float2(a.x, -a.y); }
+// Mask-gradient epilogue of the analysis (SlicqBinsParams::mask_grad, slicq_forward_mask_grad): the transform output c is
+// S^T g of an output row of the masked synthesis; instead of c the kernel stores d loss / d mask = Re(conj(X) c), X the
+// mixture coefficient that row's mask multiplied.  The mixture is only read.
+SLICQ_DEVFN float mask_grad_of(float2 x, float2 c) { return fmaf(x.x, c.x, x.y * c.y); }
 
 // ---------------------------------------------------------------------------------------
 // mirrored-bin pass of the reference (nsigtf.py:63-80) for a bin that reaches below DC: one entry per spectrum position.
@@ -275,9 +279,10 @@ struct SlicqBucketArg {
     // OUTPUT rows [targets*rows][F][S][M]; null = plain synthesis
     const float* mptr;
     // fused magnitude (slicq_forward_norm, reference: ComplexNorm transforms.py:181-208 /
-    // abs_of_real_complex phase.py:116-118): analysis also writes |c| as fp32 [rows][F][S][M]; null = off
+    // abs_of_real_complex phase.py:116-118): analysis also writes |c| as fp32 [rows][F][S][M]; null = off.
+    // Mask-gradient analysis (SlicqBinsParams::mask_grad): the fp32 mask gradient [targets*rows][F][S][M]
     float* nptr;
-    long long ms_row, ms_bin, ms_slice;   // element strides of the mask (synthesis) / magnitude (analysis) tensor
+    long long ms_row, ms_bin, ms_slice;   // element strides of the mask (synthesis) / magnitude or mask gradient (analysis)
 };
 
 struct SlicqBinsParams {
@@ -288,8 +293,11 @@ struct SlicqBinsParams {
     int rs0;               // flattened index (row * S + slice) of the first unit of the chunk
     int S;                 // slices per row in this call
     int n_buckets;
-    int x_rows;            // masked synthesis: rows of the mixture tensor (output row r reads mixture row r % x_rows); else 0
+    int x_rows;            // masked synthesis / mask-gradient analysis: rows of the mixture tensor (output row r reads
+                           // mixture row r % x_rows); else 0
     int k0;                // global index of local slice 0 (slice parity for the mirrored-bin pass)
+    int mask_grad;         // analysis: b[].ptr is the mixture (read only), b[].nptr receives Re(conj(mixture) c) instead of c
+                           // (slicq_forward_mask_grad); 0 = normal analysis
     SlicqBucketArg b[SLICQ_MAX_BUCKETS];
 };
 

@@ -79,7 +79,7 @@ struct JobCtx {
     int first_bin;
     int rs0, S;     // chunk origin and slices per row: unit g is (row, k) = divmod(rs0 + g, S)
     int x_rows;     // masked synthesis: mixture rows (0 = plain)
-    bool aux;       // a second tensor (synthesis: mask, analysis: magnitude output) is addressed through ms_*
+    bool aux;       // a second tensor (synthesis: mask, analysis: magnitude or mask-gradient output) is addressed through ms_*
 };
 
 SLICQ_DEVFN float2 cneg_if(float2 v, bool neg) { return neg ? make_float2(-v.x, -v.y) : v; }
@@ -88,14 +88,15 @@ SLICQ_DEVFN float2 cneg_if(float2 v, bool neg) { return neg ? make_float2(-v.x, 
 // element offset of (row, bin f, slice k, 0) in the caller's bucket tensor: slot = gs * F + f.
 // One integer division per slot and iteration instead of one per coefficient.
 // In masked synthesis (mixture * mask fused into the load, reference: phase.py:96-113 /
-// model.py:258-265) a second table [256, 512) holds the offsets into the mask tensor.
+// model.py:258-265) a second table [256, 512) holds the offsets into the mask tensor.  In the mask-gradient analysis
+// the first table addresses the mixture (row % x_rows) and the second the gradient (output row).
 #define SLICQ_SLOT_BYTES 4096
-SLICQ_DEVFN void fill_slot_off(long long* so, const SlicqBucketArg& b, const JobCtx& j, int base, int ng) {
+SLICQ_DEVFN void fill_slot_off(long long* so, const SlicqBucketArg& b, const JobCtx& j, int base, int ng, int x_rows) {
     for (int t = threadIdx.x; t < ng * j.F; t += blockDim.x) {
         const int gs = t / j.F, f = t - gs * j.F;
         const int rs = SLICQ_CUNIT(j.rs0 + base + gs);
         const int row = rs / j.S, k = rs - row * j.S;
-        const int rowx = j.x_rows ? row % j.x_rows : row;
+        const int rowx = x_rows ? row % x_rows : row;
         so[t] = rowx * b.s_row + f * b.s_bin + k * b.s_slice;
         if (j.aux) so[256 + t] = row * b.ms_row + f * b.ms_bin + k * b.ms_slice;
     }
@@ -106,7 +107,10 @@ SLICQ_DEVFN float cmag(float2 v) { return sqrtf(fmaf(v.x, v.x, v.y * v.y)); }
 // =========================================================================================
 // kind 1
 // =========================================================================================
-template <int M>
+// Analysis transforms: MG = mask-gradient epilogue (SlicqBinsParams::mask_grad, slicq_forward_mask_grad).  A compile-time
+// mode with a kernel of its own (bins_fwd_mask_grad_kernel): bins_fwd_kernel keeps the code and registers of the plain
+// analysis (a run-time branch in the stores cost 0.7 % of the default bench step on a B200 at 1000 W).
+template <int M, bool MG>
 SLICQ_DEVFN void ana_single(const SlicqBinsParams& p, const SlicqBucketArg& b, const JobCtx& j, float2* sm) {
     constexpr int PITCH = M + 1;
     const int tid = threadIdx.x;
@@ -139,7 +143,7 @@ SLICQ_DEVFN void ana_single(const SlicqBinsParams& p, const SlicqBucketArg& b, c
     for (int base = j.u0; base < j.u1; base += j.gt) {
         const int g = base + gs;
         const int ng = (j.u1 - base < j.gt) ? (j.u1 - base) : j.gt;
-        fill_slot_off(so, b, j, base, ng);
+        fill_slot_off(so, b, j, base, ng, MG ? p.x_rows : 0);
         if (act && g < j.u1) {
             const float4* h = reinterpret_cast<const float4*>(p.spec + (long long)g * p.spec_stride + hoff);
             float2 v[M];
@@ -158,6 +162,10 @@ SLICQ_DEVFN void ana_single(const SlicqBinsParams& p, const SlicqBucketArg& b, c
         for (int t = tid; t < ng * j.F * M; t += blockDim.x) {
             const int slot = t / M, n = t - slot * M;
             const float2 c = sm[slot * PITCH + n];
+            if (MG) {
+                b.nptr[so[256 + slot] + n] = mask_grad_of(b.ptr[so[slot] + n], c);
+                continue;
+            }
             b.ptr[so[slot] + n] = c;
             if (b.nptr != nullptr) b.nptr[so[256 + slot] + n] = cmag(c);
         }
@@ -193,7 +201,7 @@ SLICQ_DEVFN void syn_single(const SlicqBinsParams& p, const SlicqBucketArg& b, c
                      (((b.s_row | b.s_bin | b.s_slice) & 1) == 0);
     for (int base = j.u0; base < j.u1; base += j.gt) {
         const int ng = (j.u1 - base < j.gt) ? (j.u1 - base) : j.gt;
-        fill_slot_off(so, b, j, base, ng);
+        fill_slot_off(so, b, j, base, ng, j.x_rows);
         __syncthreads();
         if (vec) {
             // four independent 16-byte loads in flight per thread (a rolled loop would wait for each in turn)
@@ -258,7 +266,7 @@ SLICQ_DEVFN void syn_single(const SlicqBinsParams& p, const SlicqBucketArg& b, c
 // kind 2 : M = A * B, A >= B
 // =========================================================================================
 // analysis: x'[B*n1 + n2] -> X[k1 + A*k2];  pass 1 = DFT-A (hoisted window), pass 2 = DFT-B (runs of A to HBM)
-template <int M, int A, int B>
+template <int M, int A, int B, bool MG>
 SLICQ_DEVFN void ana_two_pass(const SlicqBinsParams& p, const SlicqBucketArg& b, const JobCtx& j, float2* sm) {
     static_assert(A * B == M, "bad split");
     constexpr int BP = (B % 2 == 0) ? B + 1 : B;
@@ -293,7 +301,7 @@ SLICQ_DEVFN void ana_two_pass(const SlicqBinsParams& p, const SlicqBucketArg& b,
         BINS_T(t0_);
         const int g = base + gs1;
         const int ng = (j.u1 - base < j.gt) ? (j.u1 - base) : j.gt;
-        fill_slot_off(so, b, j, base, ng);
+        fill_slot_off(so, b, j, base, ng, MG ? p.x_rows : 0);
         if (act1 && g < j.u1) {
             const float2* h = p.spec + (long long)g * p.spec_stride + hoff;
             float2 v[A];
@@ -319,6 +327,12 @@ SLICQ_DEVFN void ana_two_pass(const SlicqBinsParams& p, const SlicqBucketArg& b,
             for (int n = 0; n < B; ++n) v[n] = src[n];
             dft<B, true>(v);
             float2* o = b.ptr + so[slot] + k1;
+            if (MG) {
+                float* og = b.nptr + so[256 + slot] + k1;
+#pragma unroll
+                for (int k2 = 0; k2 < B; ++k2) og[A * k2] = mask_grad_of(o[A * k2], cneg_if(v[k2], (A * k2) & 1));
+                continue;
+            }
 #pragma unroll
             for (int k2 = 0; k2 < B; ++k2) o[A * k2] = cneg_if(v[k2], (A * k2) & 1);
             if (b.nptr != nullptr) {
@@ -481,7 +495,7 @@ struct PrimeDstAna {                       // analysis pass 1: output k1 -> stag
 constexpr __host__ __device__ int prime_parts(int P) { return P <= 41 ? 2 : (P <= 61 ? 3 : 4); }   // gen_codelets.py PRIME_PARTS
 
 // analysis (prime first): x'[R*n1 + n2], n1 in [0,P) -> X[k1 + P*k2]
-template <int M, int P, int R>
+template <int M, int P, int R, bool MG>
 SLICQ_DEVFN void ana_prime(const SlicqBinsParams& p, const SlicqBucketArg& b, const JobCtx& j, float* smf) {
     static_assert(P * R == M && R % 2 == 0, "bad split");
     constexpr int NP = (P <= 41 ? 2 : (P <= 61 ? 3 : 4)), RP = R + 1, PER = P * RP;
@@ -510,7 +524,7 @@ SLICQ_DEVFN void ana_prime(const SlicqBinsParams& p, const SlicqBucketArg& b, co
     __syncthreads();
     for (int base = j.u0; base < j.u1; base += j.gt) {
         const int ng = (j.u1 - base < j.gt) ? (j.u1 - base) : j.gt;
-        fill_slot_off(so, b, j, base, ng);
+        fill_slot_off(so, b, j, base, ng, MG ? p.x_rows : 0);
         // pass 1: DFT-P, task = (part, slot, n2 < R); a part's tasks fill whole warps
         const int ncol = ng * j.F * R, colp = (ncol + 31) & ~31;
         for (int t = tid; t < NP * colp; t += blockDim.x) {
@@ -536,6 +550,12 @@ SLICQ_DEVFN void ana_prime(const SlicqBinsParams& p, const SlicqBucketArg& b, co
             for (int n = 0; n < R; ++n) v[n] = cpx_ld(src + (n + R / 2) % R);
             dft<R, true>(v);
             float2* o = b.ptr + so[s] + k1;
+            if (MG) {
+                float* og = b.nptr + so[256 + s] + k1;
+#pragma unroll
+                for (int k2 = 0; k2 < R; ++k2) og[P * k2] = mask_grad_of(o[P * k2], cpx_to(v[k2]));
+                continue;
+            }
 #pragma unroll
             for (int k2 = 0; k2 < R; ++k2) cpx_st(o + P * k2, v[k2]);
             if (b.nptr != nullptr) {
@@ -583,7 +603,7 @@ SLICQ_DEVFN void syn_prime(const SlicqBinsParams& p, const SlicqBucketArg& b, co
     }
     for (int base = j.u0; base < j.u1; base += j.gt) {
         const int ng = (j.u1 - base < j.gt) ? (j.u1 - base) : j.gt;
-        fill_slot_off(so, b, j, base, ng);
+        fill_slot_off(so, b, j, base, ng, j.x_rows);
         __syncthreads();
         // pass 1: DFT-R, task = (slot, n2 < P), input runs of P from the caller's tensor; (-1)^n1 = outputs rotated by R/2
         for (int t = tid; t < ng * j.F * P; t += blockDim.x) {

@@ -423,6 +423,49 @@ class NSGT_sliced(torch.nn.Module):
                                 scratch.data_ptr(), nbytes, _BACKEND.stream(g.device))
         return out
 
+    def mask_grad_rows(self, g: torch.Tensor, mix: Sequence[torch.Tensor], n_targets: int,
+                       lead=None) -> List[torch.Tensor]:
+        """Gradient of ``backward_rows_masked`` with respect to its masks.  g [T * N, length] (gradient w.r.t. that
+        call's output, row t * N + n), mix: the per-bucket complex [N, F_b, S, M_b] mixture it read (any strides, M
+        contiguous).  Returns per bucket float32 [T * N, F_b, S, M_b] (or [*lead, F_b, S, M_b]), one slab as
+        ``alloc_norms``: Re(conj(mix[n]) * (S^T g)[t * N + n]).  The adjoint of the synthesis runs on the analysis
+        kernels of the ``synthesis_adjoint_rows`` plan, whose epilogue takes the product with the mixture: S^T g is never
+        stored."""
+        _BACKEND.check(g)
+        t = self.tables
+        if len(mix) != len(t.buckets):
+            raise ValueError(f"expected {len(t.buckets)} buckets")
+        if self._adj_tables is None:
+            self._adj_tables = _AdjointTables(self.tables)
+        if g.dtype != torch.float32:
+            g = g.to(torch.float32)
+        if g.stride(1) != 1:
+            g = g.contiguous()
+        Tn = int(n_targets)
+        N, S = mix[0].shape[0], mix[0].shape[2]
+        if g.shape[0] != Tn * N:
+            raise ValueError(f"expected {Tn * N} gradient rows, got {g.shape[0]}")
+        vx, keep = [], []
+        for c, (_, nb, M) in zip(mix, t.buckets):
+            if c.dtype != torch.complex64:
+                c = c.to(torch.complex64)
+            if tuple(c.shape) != (N, nb, S, M):
+                raise ValueError(f"bucket shape {tuple(c.shape)} != {(N, nb, S, M)}")
+            if c.stride(3) != 1:
+                c = c.contiguous()
+            keep.append(c)
+            vx.append(self._view_of(c))
+        plan = self._adj_cache.get(self._adj_tables, g.device)
+        with _BACKEND.device_guard(g.device):
+            slab, out = self.alloc_norms(Tn * N, S, g.device, lead=lead)
+            vg = [(o.data_ptr(), nb * S * M, S * M, M) for o, (_, nb, M) in zip(out, t.buckets)]
+            nbytes = plan.scratch_bytes(Tn * N, S, False)
+            scratch = torch.empty(nbytes, dtype=torch.uint8, device=g.device)
+            plan.forward_mask_grad(g.data_ptr(), Tn, N, g.stride(0), g.shape[1], 0, 0, S, vx, vg,
+                                   scratch.data_ptr(), nbytes, _BACKEND.stream(g.device))
+        del keep
+        return out
+
     def analysis_adjoint_views(self, views, n_rows: int, n_slices: int, device, length: int) -> torch.Tensor:
         """Gradient of the analysis: per-bucket views of d [N, F_b, S, M_b] complex (gradient w.r.t. the coefficients) ->
         [N, length] float32 = A^T d, the transpose of ``forward_rows`` with respect to the real inner products

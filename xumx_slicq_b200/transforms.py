@@ -231,7 +231,14 @@ class INSGT_SL(nn.Module):
         """Fused realtime-model synthesis (not in the reference API; SURVEY.md section 8 row A10):
         X_list per bucket [B, C, F, S, M, 2] (the mixture sliCQT), mask_list per bucket
         [targets, B, C, F, S, M] (the CDAE sigmoid masks, model.py:231-234).  Returns
-        [targets, B, C, length] == self.forward([m.unsqueeze(-1) * X for ...], length)."""
+        [targets, B, C, length] == self.forward([m.unsqueeze(-1) * X for ...], length).
+        Differentiable with respect to the masks and X (:class:`_MaskedInverseFn`)."""
+        if torch.is_grad_enabled() and any(t.requires_grad for t in list(X_list) + list(mask_list)):
+            return _MaskedInverseFn.apply(self, length, len(X_list), *X_list, *mask_list)
+        return self._forward_masked_impl(X_list, mask_list, length)
+
+    def _masked_inputs(self, X_list, mask_list):
+        """(mixture per bucket complex [N, F, S, M], masks per bucket [targets, N, F, S, M], lead dims of X)."""
         dev = _module_device(self.nsgt)
         xs, ms = [], []
         lead = None
@@ -246,8 +253,59 @@ class INSGT_SL(nn.Module):
             lead = tuple(Xc.shape[:-3])
             xs.append(Xc.reshape((-1,) + tuple(Xc.shape[-3:])))
             ms.append(Mk.reshape((Mk.shape[0], -1) + tuple(Mk.shape[-3:])))
+        return xs, ms, lead
+
+    def _forward_masked_impl(self, X_list, mask_list, length: int) -> Tensor:
+        xs, ms, lead = self._masked_inputs(X_list, mask_list)
         y = self.nsgt.nsgt.backward_rows_masked(xs, ms, length)
         return y.view(ms[0].shape[0], *lead, -1)
+
+
+class _MaskedInverseFn(torch.autograd.Function):
+    """Differentiable fused masked synthesis.  Output row r = t * N + n is y_r = S(m_r * X_n), so with g_r = dL/dy_r
+        dL/dm_r = Re(conj(X_n) * S^T g_r),        dL/dX_n = sum_t m_{t,n} * S^T g_{t*N+n}.
+    When only masks need a gradient, one call of the adjoint-of-synthesis analysis kernels takes the product with the
+    mixture in their epilogue (NSGT_sliced.mask_grad_rows): S^T g is never stored.  When X needs one, S^T g is computed
+    once (synthesis_adjoint_rows) and both products are taken in torch."""
+
+    @staticmethod
+    def forward(ctx, module, length, n, *tensors):
+        ctx.module, ctx.length, ctx.n = module, length, n
+        ctx.save_for_backward(*tensors)
+        with torch.no_grad():
+            return module._forward_masked_impl(list(tensors[:n]), list(tensors[n:]), length)
+
+    @staticmethod
+    def backward(ctx, gy):
+        module, n = ctx.module, ctx.n
+        nsg = module.nsgt.nsgt
+        saved = ctx.saved_tensors
+        X_list, mask_list = saved[:n], saved[n:]
+        need_x, need_m = ctx.needs_input_grad[3:3 + n], ctx.needs_input_grad[3 + n:]
+        xs, ms, lead = module._masked_inputs(X_list, mask_list)
+        Tn, N = ms[0].shape[0], xs[0].shape[0]
+        S = xs[0].shape[2]
+        g = gy.reshape(Tn * N, gy.shape[-1])
+        gx, gm = [None] * n, [None] * n
+        if any(need_x):
+            cadj = nsg.synthesis_adjoint_rows(g, S)                  # per bucket complex [T * N, F, S, M]
+            for i, (c, x, m) in enumerate(zip(cadj, xs, ms)):
+                c = c.view((Tn, N) + tuple(c.shape[1:]))
+                if need_x[i]:
+                    d = (c * m.to(torch.float32)).sum(0)
+                    gx[i] = torch.view_as_real(d).reshape(X_list[i].shape).to(X_list[i].dtype)
+                if need_m[i]:
+                    gm[i] = torch.real(x.conj() * c)
+        elif any(need_m):
+            gm = nsg.mask_grad_rows(g, xs, Tn)
+        for i in range(n):
+            if not need_m[i]:
+                gm[i] = None
+            elif gm[i] is not None:
+                gm[i] = gm[i].reshape(mask_list[i].shape).to(device=mask_list[i].device, dtype=mask_list[i].dtype)
+            if gx[i] is not None:
+                gx[i] = gx[i].to(device=X_list[i].device)
+        return (None, None, None) + tuple(gx) + tuple(gm)
 
 
 class ComplexNorm(nn.Module):
