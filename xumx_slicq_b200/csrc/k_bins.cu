@@ -29,40 +29,40 @@ SLICQ_DEVFN int find_bucket(const SlicqBinsParams& p, int job) {
     return lo;
 }
 
-// MG: mask-gradient epilogue of the analysis (see slicq_fft_tile.cuh); unused by the synthesis
-template <int M, int KIND, int A, int B, bool SYNTH, bool MG> struct JobRunner;
-template <int M, int A, int B, bool MG> struct JobRunner<M, 1, A, B, false, MG> {
+// MG: mask-gradient epilogue of the analysis, OVR: overflow over several runs in the synthesis (see slicq_fft_tile.cuh)
+template <int M, int KIND, int A, int B, bool SYNTH, bool MG, bool OVR> struct JobRunner;
+template <int M, int A, int B, bool MG, bool OVR> struct JobRunner<M, 1, A, B, false, MG, OVR> {
     static SLICQ_DEVFN void run(const SlicqBinsParams& p, const SlicqBucketArg& b, const JobCtx& j, unsigned char* sm) {
         ana_single<M, MG>(p, b, j, reinterpret_cast<float2*>(sm));
     }
 };
-template <int M, int A, int B, bool MG> struct JobRunner<M, 1, A, B, true, MG> {
+template <int M, int A, int B, bool MG, bool OVR> struct JobRunner<M, 1, A, B, true, MG, OVR> {
     static SLICQ_DEVFN void run(const SlicqBinsParams& p, const SlicqBucketArg& b, const JobCtx& j, unsigned char* sm) {
         syn_single<M>(p, b, j, reinterpret_cast<float2*>(sm));
     }
 };
-template <int M, int A, int B, bool MG> struct JobRunner<M, 2, A, B, false, MG> {
+template <int M, int A, int B, bool MG, bool OVR> struct JobRunner<M, 2, A, B, false, MG, OVR> {
     static SLICQ_DEVFN void run(const SlicqBinsParams& p, const SlicqBucketArg& b, const JobCtx& j, unsigned char* sm) {
         ana_two_pass<M, A, B, MG>(p, b, j, reinterpret_cast<float2*>(sm));
     }
 };
-template <int M, int A, int B, bool MG> struct JobRunner<M, 2, A, B, true, MG> {
+template <int M, int A, int B, bool MG, bool OVR> struct JobRunner<M, 2, A, B, true, MG, OVR> {
     static SLICQ_DEVFN void run(const SlicqBinsParams& p, const SlicqBucketArg& b, const JobCtx& j, unsigned char* sm) {
-        syn_two_pass<M, A, B>(p, b, j, reinterpret_cast<float2*>(sm));
+        syn_two_pass<M, A, B, OVR>(p, b, j, reinterpret_cast<float2*>(sm));
     }
 };
-template <int M, int A, int B, bool MG> struct JobRunner<M, 3, A, B, false, MG> {
+template <int M, int A, int B, bool MG, bool OVR> struct JobRunner<M, 3, A, B, false, MG, OVR> {
     static SLICQ_DEVFN void run(const SlicqBinsParams& p, const SlicqBucketArg& b, const JobCtx& j, unsigned char* sm) {
         ana_prime<M, A, B, MG>(p, b, j, reinterpret_cast<float*>(sm));
     }
 };
-template <int M, int A, int B, bool MG> struct JobRunner<M, 3, A, B, true, MG> {
+template <int M, int A, int B, bool MG, bool OVR> struct JobRunner<M, 3, A, B, true, MG, OVR> {
     static SLICQ_DEVFN void run(const SlicqBinsParams& p, const SlicqBucketArg& b, const JobCtx& j, unsigned char* sm) {
-        syn_prime<M, A, B>(p, b, j, reinterpret_cast<float*>(sm));
+        syn_prime<M, A, B, OVR>(p, b, j, reinterpret_cast<float*>(sm));
     }
 };
 
-template <bool SYNTH, bool MG>
+template <bool SYNTH, bool MG, bool OVR>
 SLICQ_DEVFN void bins_body(const SlicqBinsParams& p, unsigned char* smem) {
     const int job = blockIdx.x;
     const int bi = find_bucket(p, job);
@@ -86,7 +86,7 @@ SLICQ_DEVFN void bins_body(const SlicqBinsParams& p, unsigned char* smem) {
     }
     switch (b.M) {
 #define SLICQ_FFT_SIZE(M_, K_, A_, B_, C_) \
-    case M_: JobRunner<M_, K_, A_, B_, SYNTH, MG>::run(p, b, j, smem); break;
+    case M_: JobRunner<M_, K_, A_, B_, SYNTH, MG, OVR>::run(p, b, j, smem); break;
 #include "fft_sizes.inc"
 #undef SLICQ_FFT_SIZE
         default: break;
@@ -104,24 +104,31 @@ SLICQ_DEVFN void bins_body(const SlicqBinsParams& p, unsigned char* smem) {
 
 __global__ void __launch_bounds__(SLICQ_BINS_THREADS, SLICQ_BINS_MIN_BLOCKS) bins_fwd_kernel(const __grid_constant__ SlicqBinsParams p) {
     SLICQ_DYN_SMEM(unsigned char, smem);
-    bins_body<false, false>(p, smem);
+    bins_body<false, false, false>(p, smem);
 }
 
 // the analysis with the mask-gradient epilogue (SlicqBinsParams::mask_grad): the adjoint-of-synthesis plan's
 // slicq_forward_mask_grad
 __global__ void __launch_bounds__(SLICQ_BINS_THREADS, SLICQ_BINS_MIN_BLOCKS) bins_fwd_mask_grad_kernel(const __grid_constant__ SlicqBinsParams p) {
     SLICQ_DYN_SMEM(unsigned char, smem);
-    bins_body<false, true>(p, smem);
+    bins_body<false, true, false>(p, smem);
 }
 
 __global__ void __launch_bounds__(SLICQ_BINS_THREADS, SLICQ_BINS_MIN_BLOCKS) bins_inv_kernel(const __grid_constant__ SlicqBinsParams p) {
     SLICQ_DYN_SMEM(unsigned char, smem);
-    bins_body<true, false>(p, smem);
+    bins_body<true, false, false>(p, smem);
+}
+
+// the synthesis for plans whose two-pass or prime bins divert more than their first run of outputs to the overflow slot
+// (slicq_plan::ov_multi_run: the lowest bins of some Bark / mel filterbanks with few bins or a low fmin)
+__global__ void __launch_bounds__(SLICQ_BINS_THREADS, SLICQ_BINS_MIN_BLOCKS) bins_inv_ovr_kernel(const __grid_constant__ SlicqBinsParams p) {
+    SLICQ_DYN_SMEM(unsigned char, smem);
+    bins_body<true, false, true>(p, smem);
 }
 
 extern "C" int slicq_bins_threads(void) { return SLICQ_BINS_THREADS; }
 
-// host-side launcher (called from slicq_api.cu) -----------------------------------------------
+// host-side launcher (called from slicq_api.cu); synth: 0 analysis, 1 synthesis, 2 synthesis with overflow over several runs
 extern "C" int slicq_launch_bins(const SlicqBinsParams* p, int n_jobs, int smem_bytes, int synth, cudaStream_t s) {
     if (n_jobs <= 0) return 0;
 #ifndef SLICQ_EMU
@@ -133,11 +140,14 @@ extern "C" int slicq_launch_bins(const SlicqBinsParams* p, int n_jobs, int smem_
             if (SLICQ_SET_SMEM(bins_fwd_kernel, 100 * 1024) != cudaSuccess) return -3;
             if (SLICQ_SET_SMEM(bins_inv_kernel, 100 * 1024) != cudaSuccess) return -3;
             if (SLICQ_SET_SMEM(bins_fwd_mask_grad_kernel, 100 * 1024) != cudaSuccess) return -3;
+            if (SLICQ_SET_SMEM(bins_inv_ovr_kernel, 100 * 1024) != cudaSuccess) return -3;
             if (dev >= 0 && dev < 64) done[dev] = true;
         }
     }
 #endif
-    if (synth) {
+    if (synth == 2) {
+        SLICQ_LAUNCH(bins_inv_ovr_kernel, dim3(n_jobs), dim3(SLICQ_BINS_THREADS), smem_bytes, s, *p);
+    } else if (synth) {
         SLICQ_LAUNCH(bins_inv_kernel, dim3(n_jobs), dim3(SLICQ_BINS_THREADS), smem_bytes, s, *p);
     } else if (p->mask_grad) {
         SLICQ_LAUNCH(bins_fwd_mask_grad_kernel, dim3(n_jobs), dim3(SLICQ_BINS_THREADS), smem_bytes, s, *p);

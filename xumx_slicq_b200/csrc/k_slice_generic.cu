@@ -126,13 +126,16 @@ __global__ void __launch_bounds__(SLICQ_GEN_THREADS, 1) slice_fft_inv_generic_ke
         const float2 a = __ldg(P0 + f), b = __ldg(P1 + f);
         A[f] = make_float2(a.x + b.x, a.y + b.y);
     }
-    __syncthreads();
-    for (int i = tid; i < p.t.n_ex; i += NT) {
-        const int4 q = __ldg(p.t.ex + i);
-        if (q.w) continue;                      // folded entries: below
-        float2 e = __ldg(Trow + q.y);
-        if (q.z >= 0) { const float2 v = __ldg(Trow + q.z); e.x += v.x; e.y += v.y; }
-        A[q.x].x += e.x; A[q.x].y += e.y;
+    // overflow entries round by round: the targets of one round are distinct, a barrier orders the rounds
+    for (int r = 0; r < p.t.ex_rounds; ++r) {
+        __syncthreads();
+        for (int i = tid; i < p.t.n_ex; i += NT) {
+            const int4 q = __ldg(p.t.ex + i);
+            if (q.w != 2 * r) continue;             // other rounds; folded entries: below
+            float2 e = __ldg(Trow + q.y);
+            if (q.z >= 0) { const float2 v = __ldg(Trow + q.z); e.x += v.x; e.y += v.y; }
+            A[q.x].x += e.x; A[q.x].y += e.y;
+        }
     }
     if (p.t.adjoint & 2) {
         __syncthreads();
@@ -145,14 +148,17 @@ __global__ void __launch_bounds__(SLICQ_GEN_THREADS, 1) slice_fft_inv_generic_ke
             A[N - f].x += a.x + b.x; A[N - f].y -= a.y + b.y;
         }
         // overflow entries below DC / above Nyquist fold back conjugated, like the plane margins above: their targets
-        // coincide with those of the margins and of the direct entries, so in a pass of their own (distinct targets)
-        __syncthreads();
-        for (int i = tid; i < p.t.n_ex; i += NT) {
-            const int4 q = __ldg(p.t.ex + i);
-            if (!q.w) continue;
-            float2 e = __ldg(Trow + q.y);
-            if (q.z >= 0) { const float2 v = __ldg(Trow + q.z); e.x += v.x; e.y += v.y; }
-            A[q.x].x += e.x; A[q.x].y -= e.y;
+        // coincide with those of the margins and of the direct entries, so in a pass of their own (distinct targets
+        // within a round)
+        for (int r = 0; r < p.t.ex_rounds; ++r) {
+            __syncthreads();
+            for (int i = tid; i < p.t.n_ex; i += NT) {
+                const int4 q = __ldg(p.t.ex + i);
+                if (q.w != 2 * r + 1) continue;
+                float2 e = __ldg(Trow + q.y);
+                if (q.z >= 0) { const float2 v = __ldg(Trow + q.z); e.x += v.x; e.y += v.y; }
+                A[q.x].x += e.x; A[q.x].y -= e.y;
+            }
         }
     }
     __syncthreads();

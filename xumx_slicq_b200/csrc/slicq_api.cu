@@ -4,6 +4,7 @@
 //            (slicq_forward_mask_grad: the same sequence, bins_fwd_kernel / mirror_adj_kernel in their mask-gradient mode)
 // inverse  : per chunk                         bins_inv_kernel [-> mirror_fix_kernel] -> slice_fft_inv_kernel (even slices,
 //                                              then odd slices)
+//            (bins_inv_ovr_kernel in place of bins_inv_kernel for plans whose overflow spans several transform runs)
 // (the bracketed kernels only for bins that reach below DC; mirror_adj_kernel only in the adjoint-of-synthesis plan)
 // A chunk's intermediate spectra (analysis: padded half spectra H; synthesis: the two bin planes T) live in the
 // caller-provided scratch buffer; SLICQ_CHUNK_MB bounds the chunk (default: one chunk per call).
@@ -153,6 +154,7 @@ struct slicq_plan {
     SlicqDeviceTables dev;
     std::vector<void*> owned;
     int bins_smem;        // dynamic shared memory of the bins kernels
+    bool ov_multi_run;    // a two-pass / prime bin diverts more than its first run of outputs: synthesis by bins_inv_ovr_kernel
     int pad_l, pad_r;
     long long spec_stride_fwd;
     long long t_stride;   // complex elements per unit of the synthesis intermediate T
@@ -235,9 +237,10 @@ extern "C" int slicq_plan_create(const slicq_tables* t, slicq_plan** out) {
             delete p;
             return fail(SLICQ_E_UNSUPPORTED, "bin length M must be a multiple of 4 in [16, 292]");
         }
-        if (pos % 2 != 0 || pos < 0 || pos > p->N2 || (j > 0 && pos <= p->bin_pos[j - 1])) {
+        // the lowest bins of Bark / mel filterbanks with few bins or a low fmin can share a position
+        if (pos % 2 != 0 || pos < 0 || pos > p->N2 || (j > 0 && pos < p->bin_pos[j - 1])) {
             delete p;
-            return fail(SLICQ_E_UNSUPPORTED, "bin positions must be even, increasing and within [0, L/2]");
+            return fail(SLICQ_E_UNSUPPORTED, "bin positions must be even, non-decreasing and within [0, L/2]");
         }
         p->bin_coff[j] = off;
         off += M;
@@ -332,32 +335,38 @@ extern "C" int slicq_plan_create(const slicq_tables* t, slicq_plan** out) {
     const int N2 = p->N2;
     const int pl_off = pad_l;                                            // even
     const int pl_len = (pl_off + N2 + 2 + std::max(pad_r, 2) + 1) & ~1;  // positions -pl_off .. N2 + 1 + pad_r, even
+    // Bin j writes positions [lo_j + ov_j, lo_j + M_j) of its plane.  Its leading ov_j positions, those that an earlier bin
+    // of the plane already reaches (the furthest end of all of them, clamped to the bin), go to its overflow slot: every
+    // plane position has at most one writer.  ov_j is even (positions and half lengths are), and may be all of M_j.
     std::vector<int> toff(J), ov(J, 0), ovoff(J, 0);
     int n_ovf = 0;
+    int plane_end[2] = {-2 * N2 - 2, -2 * N2 - 2};
     for (int j = 0; j < J; ++j) {
         const int lo = p->bin_pos[j] - p->bin_M[j] / 2;
         toff[j] = (j & 1) * pl_len + pl_off + lo;
-        if (j >= 2) {
-            const int end_prev = p->bin_pos[j - 2] + p->bin_M[j - 2] / 2;
-            ov[j] = std::max(0, end_prev - lo);
-        }
-        if (ov[j] > p->bin_M[j] || (ov[j] & 1)) { delete p; return fail(SLICQ_E_UNSUPPORTED, "unsupported overlap between bins of one plane"); }
-        if (j >= 4 && p->bin_pos[j - 4] + p->bin_M[j - 4] / 2 > lo) { delete p; return fail(SLICQ_E_UNSUPPORTED, "more than 4 bins overlap at one spectrum position"); }
+        ov[j] = std::min(p->bin_M[j], std::max(0, plane_end[j & 1] - lo));
+        plane_end[j & 1] = std::max(plane_end[j & 1], lo + p->bin_M[j]);
         ovoff[j] = 2 * pl_len + n_ovf;
         n_ovf += ov[j];
     }
-    // two-pass / prime transforms store their first run of A outputs through one select: the overflow part must fit
+    // two-pass / prime transforms divert only their first run of outputs (A, resp. R = B) to the overflow slot, through one
+    // select; a plan with a longer overflow runs the synthesis variant that checks every output (bins_inv_ovr_kernel)
+    p->ov_multi_run = false;
     for (const Bucket& b : p->buckets)
         for (int j = b.first_bin; j < b.first_bin + b.n_bins; ++j)
-            if ((b.kind == 2 && ov[j] > b.A) || (b.kind == 3 && ov[j] > b.B)) { delete p; return fail(SLICQ_E_UNSUPPORTED, "overlap between bins of one plane exceeds the first transform pass"); }
+            if ((b.kind == 2 && ov[j] > b.A) || (b.kind == 3 && ov[j] > b.B)) p->ov_multi_run = true;
     p->t_stride = (2LL * pl_len + n_ovf + 1) & ~1LL;
-    // overflow entries, one per target position.  The synthesis drops the parts outside [0, N2]; the adjoint of the analysis
-    // folds them back conjugated (the analysis reads the Hermitian mirror there), as separate entries after the direct ones:
-    // their targets may coincide with direct targets, so the slice kernel adds them in a later pass
+    // overflow entries {f, off0, off1 or -1, fold | round << 1}: position f also receives T[off0] (+ T[off1]).  The synthesis
+    // drops the parts outside [0, N2]; the adjoint of the analysis folds them back conjugated (the analysis reads the
+    // Hermitian mirror there), as separate entries after the direct ones: their targets may coincide with direct targets,
+    // so the slice kernel adds them in a later pass.  The slots of one position, in bin order, pair up into entries; the
+    // r-th entry of every position belongs to round r, so the targets of a round are distinct and the slice kernel adds
+    // the rounds one after the other (a barrier in between, no atomics).  Entries are ordered by (fold, round, f).
     std::vector<int4> ex;
+    int ex_rounds = 0;
     {
         const bool fold = (t->flags & SLICQ_PLAN_ADJOINT_OF_ANALYSIS) != 0;
-        std::vector<int> e0(N2 + 1, -1), e1(N2 + 1, -1), c0(N2 + 1, -1), c1(N2 + 1, -1);
+        std::vector<std::vector<int> > slots[2] = {std::vector<std::vector<int> >(N2 + 1), std::vector<std::vector<int> >(N2 + 1)};
         for (int j = 0; j < J; ++j)
             for (int m = 0; m < ov[j]; ++m) {
                 int f = p->bin_pos[j] - p->bin_M[j] / 2 + m;
@@ -365,44 +374,55 @@ extern "C" int slicq_plan_create(const slicq_tables* t, slicq_plan** out) {
                 if (out && !fold) continue;
                 if (f < 0) f = -f;
                 if (f > N2) f = 2 * N2 - f;
-                std::vector<int>& a = out ? c0 : e0;
-                std::vector<int>& b = out ? c1 : e1;
-                if (a[f] < 0) a[f] = ovoff[j] + m;
-                else if (b[f] < 0) b[f] = ovoff[j] + m;
-                else { delete p; return fail(SLICQ_E_UNSUPPORTED, "more than two overflow entries at one spectrum position"); }
+                slots[out][f].push_back(ovoff[j] + m);
             }
-        for (int f = 0; f <= N2; ++f)
-            if (e0[f] >= 0) ex.push_back(int4{f, e0[f], e1[f], 0});
-        for (int f = 0; f <= N2; ++f)
-            if (c0[f] >= 0) ex.push_back(int4{f, c0[f], c1[f], 1});
-        // the tuned slice kernels (k_slice.cu) have no folded pass
+        for (int w = 0; w < 2; ++w) {
+            size_t most = 0;
+            for (const std::vector<int>& s : slots[w]) most = std::max(most, s.size());
+            const int rounds = (int)((most + 1) / 2);
+            ex_rounds = std::max(ex_rounds, rounds);
+            for (int r = 0; r < rounds; ++r)
+                for (int f = 0; f <= N2; ++f) {
+                    const std::vector<int>& s = slots[w][f];
+                    if ((int)s.size() > 2 * r) ex.push_back(int4{f, s[2 * r], (int)s.size() > 2 * r + 1 ? s[2 * r + 1] : -1, w | (r << 1)});
+                }
+        }
+        // the tuned slice kernels (k_slice.cu) have no folded pass and add the entries in one round
         if (L == kTunedSliceLen && ex.size() > 0 && ex.back().w) {
             delete p;
             return fail(SLICQ_E_UNSUPPORTED, "adjoint of the analysis: overflow below DC / above Nyquist is not implemented in "
+                                             "the tuned slice kernels (slice length 18060)");
+        }
+        if (L == kTunedSliceLen && ex_rounds > 1) {
+            delete p;
+            return fail(SLICQ_E_UNSUPPORTED, "more than two overflow entries at one spectrum position are not implemented in "
                                              "the tuned slice kernels (slice length 18060)");
         }
     }
     const int n_ex = (int)ex.size();
     if (ex.empty()) ex.push_back(int4{0, 0, -1, 0});
     // gaps: positions of a plane row (-pl_off .. pl_len - pl_off - 1, margins included: the adjoint-of-analysis mode folds
-    // them back) that none of its bins covers; owner = the next bin of the plane (or its last)
+    // them back) that none of its bins writes (a position a bin diverts to its overflow slot is written only if another bin
+    // of the plane writes it); owner = the bin covering the next written position (or the plane's last bin)
     std::vector<int2> gaps;
     {
         std::vector<std::vector<int2> > per_bucket(p->buckets.size());
         auto bucket_of = [&](int j) { for (size_t i = 0; i < p->buckets.size(); ++i) if (j >= p->buckets[i].first_bin && j < p->buckets[i].first_bin + p->buckets[i].n_bins) return (int)i; return 0; };
         for (int q = 0; q < 2; ++q) {
             std::vector<int> owner(pl_len, -1);    // covering bin or -1, index = pl_off + f
+            std::vector<char> written(pl_len, 0);
             int last = -1;
             for (int j = q; j < J; j += 2) {
                 const int lo = std::max(0, pl_off + p->bin_pos[j] - p->bin_M[j] / 2), hi = std::min(pl_len, pl_off + p->bin_pos[j] + p->bin_M[j] / 2);
                 for (int f = lo; f < hi; ++f) owner[f] = j;
+                for (int f = std::max(lo, pl_off + p->bin_pos[j] - p->bin_M[j] / 2 + ov[j]); f < hi; ++f) written[f] = 1;
                 last = j;
             }
             if (last < 0) { delete p; return fail(SLICQ_E_UNSUPPORTED, "a bin plane is empty"); }
             for (int f = 0; f < pl_len;) {
-                if (owner[f] >= 0) { ++f; continue; }
+                if (written[f]) { ++f; continue; }
                 int g = f;
-                while (g < pl_len && owner[g] < 0) ++g;
+                while (g < pl_len && !written[g]) ++g;
                 const int next = g < pl_len ? owner[g] : last;
                 per_bucket[bucket_of(next)].push_back(int2{q * pl_len + f, g - f});
                 f = g;
@@ -487,7 +507,7 @@ extern "C" int slicq_plan_create(const slicq_tables* t, slicq_plan** out) {
     d.n_mir = n_mir; d.n_fac = (int)fac.size();
     d.n_mir_bins = n_mir_bins; d.mir_nf = mir_nf; d.mir_nc = mir_nc;
     for (size_t i = 0; i < fac.size(); ++i) d.fac[i] = fac[i];
-    d.n_ex = n_ex; d.pl_off = pl_off; d.pl_len = pl_len; d.t_stride = (int)p->t_stride;
+    d.n_ex = n_ex; d.ex_rounds = ex_rounds; d.pl_off = pl_off; d.pl_len = pl_len; d.t_stride = (int)p->t_stride;
     if (rc) {
         slicq_plan_destroy(p);
         return fail(SLICQ_E_CUDA, "device table upload failed");
@@ -518,6 +538,18 @@ extern "C" int slicq_plan_create(const slicq_tables* t, slicq_plan** out) {
     *out = p;
     return SLICQ_OK;
 }
+
+#ifdef SLICQ_EMU
+// emulation build only (tests/emu): the synthesis layout the plan derived, for tests of the plan rules.  The emulated
+// device tables are host memory.
+extern "C" int slicq_emu_plan_layout(const slicq_plan* p, const int** ov, const int4** ex, int* n_ex, int* ex_rounds,
+                                     int* ov_multi_run) {
+    if (!p) return SLICQ_E_INVALID;
+    *ov = p->dev.bin_ov; *ex = p->dev.ex; *n_ex = p->dev.n_ex; *ex_rounds = p->dev.ex_rounds;
+    *ov_multi_run = p->ov_multi_run ? 1 : 0;
+    return SLICQ_OK;
+}
+#endif
 
 extern "C" int slicq_plan_n_buckets(const slicq_plan* p) { return p ? (int)p->buckets.size() : SLICQ_E_INVALID; }
 
@@ -858,7 +890,7 @@ int inverse_one(const slicq_plan* p, const slicq_bucket_view* buckets, const sli
         while (n > 1 && u0 + n < units && ((u0 + n) % n_slices) != 0 && (((u0 + n) % n_slices) & 1) == 0) --n;
         bp->n_rs = (int)n; bp->rs0 = (int)u0;
         const int jobs = fill_bins_params(p, buckets, *bp, (int)n, masks);
-        { ProfScope ps(K_BINS_INV, s); rc = slicq_launch_bins(bp, jobs, p->bins_smem, 1, s); }
+        { ProfScope ps(K_BINS_INV, s); rc = slicq_launch_bins(bp, jobs, p->bins_smem, p->ov_multi_run ? 2 : 1, s); }
         ++g_launches;
         if (rc) break;
         if (p->dev.n_mir > 0) {          // mirrored-bin pass of configurations whose first bins reach below DC

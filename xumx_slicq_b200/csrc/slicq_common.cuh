@@ -235,17 +235,19 @@ struct SlicqDeviceTables {
     const float2* post_tw;  // [N2/2 + 1]  exp(-2 pi i k / L)
     const float2* tw;       // concatenated per-bucket twiddles exp(-2 pi i j / M_b), j in [0, M_b)
     // synthesis intermediate T, one row per unit: [plane 0][plane 1][overflow].  Plane q holds the windowed spectra
-    // of the bins j with j % 2 == q at their spectrum positions (index pl_off + f); where two bins of one plane
-    // overlap (a few positions) the leading part of the later bin goes to the overflow area instead, and the
-    // few positions no bin of a plane covers ("gaps") are zero-filled by the bins kernel.
+    // of the bins j with j % 2 == q at their spectrum positions (index pl_off + f); where a bin overlaps earlier bins of
+    // its plane, its leading part (up to all of it) goes to the overflow area instead, and the positions no bin of a
+    // plane writes ("gaps") are zero-filled by the bins kernel.
     int pl_off, pl_len;           // plane q starts at q * pl_len; position f sits at q * pl_len + pl_off + f  (both even)
     int t_stride;                 // complex elements per row of T (even)
     const int* bin_toff;          // [J] offset in the row of coefficient m' = 0 of bin j
     const int* bin_ov;            // [J] leading coefficients of bin j that go to the overflow area (even, usually 0)
     const int* bin_ovoff;         // [J] offset in the row of the overflow slot of m' = 0
-    const int4* ex;               // [n_ex] {f, off0, off1 or -1, fold}: position f also receives T[off0] (+ T[off1]),
-                                  // conjugated if fold (adjoint of the analysis: overflow below DC / above Nyquist)
+    const int4* ex;               // [n_ex] {f, off0, off1 or -1, fold | round << 1}: position f also receives T[off0]
+                                  // (+ T[off1]), conjugated if fold (adjoint of the analysis: overflow below DC / above
+                                  // Nyquist); the entries of one round have distinct f
     int n_ex;
+    int ex_rounds;                // rounds of the direct and of the folded entries (at most); 1 for most plans
     const int2* gaps;             // {offset in the row, count}: zero-filled per unit by the job of the owning bucket
     // generic slice kernels (k_slice_generic.cu): prime factors of N2 and exp(-2 pi i k / N2)
     int n_fac;

@@ -352,7 +352,9 @@ SLICQ_DEVFN void ana_two_pass(const SlicqBinsParams& p, const SlicqBucketArg& b,
 // synthesis: x[B*n1 + n2] -> X[k1 + A*k2];  same shape as the analysis: pass 1 = DFT-A with the
 // thread's (unit, bin, n2) fixed for the whole job (runs of B from the caller's tensor), pass 2 =
 // DFT-B, dual window, runs of A into the packed row T.
-template <int M, int A, int B>
+// OVR: a bin may divert more than its first run of outputs to its overflow slot (bins_inv_ovr_kernel, plans whose bins
+// crowd together near DC); a compile-time mode, so that bins_inv_kernel keeps its one select on the first run.
+template <int M, int A, int B, bool OVR>
 SLICQ_DEVFN void syn_two_pass(const SlicqBinsParams& p, const SlicqBucketArg& b, const JobCtx& j, float2* sm) {
     static_assert(A * B == M, "bad split");
     constexpr int BP = (B % 2 == 0) ? B + 1 : B;
@@ -448,7 +450,16 @@ SLICQ_DEVFN void syn_two_pass(const SlicqBinsParams& p, const SlicqBucketArg& b,
                 for (int k2 = 0; k2 < B; ++k2) oc[k2 * nt] = make_float2(v[k2].x * wp[A * k2], v[k2].y * wp[A * k2]);
                 continue;
             }
-            // overflow counts never exceed A (checked by slicq_plan_create): only output k2 = 0 can be diverted
+            if (OVR) {   // any output k1 + A k2 below the overflow count goes to the overflow slot
+#pragma unroll
+                for (int k2 = 0; k2 < B; ++k2) {
+                    const float w = wp[A * k2];
+                    float2* ok = (k1 + A * k2 < c.z) ? row + c.w + k1 + A * k2 : o + A * k2;
+                    *ok = make_float2(v[k2].x * w, v[k2].y * w);
+                }
+                continue;
+            }
+            // without OVR overflow counts never exceed A (slicq_plan_create): only output k2 = 0 can be diverted
             {
                 const float w = wp[0];
                 float2* o0 = (k1 < c.z) ? row + c.w + k1 : o;
@@ -487,6 +498,10 @@ struct PrimeSrcAna {                       // analysis pass 1: x'[R n + n2] * wi
 struct PrimeDstSyn {                       // synthesis pass 2: output k2 -> T[base + R k2] * window
     float2* o; const float* w; int R; int ovd;    // ovd: offset of the overflow slot relative to the plane slot, 0 = none
     SLICQ_DEVFN void st(int k, cpx v) const { cpx_st(o + R * k + (k == 0 ? ovd : 0), cmulr(v, w[R * k])); }
+};
+struct PrimeDstSynOvr {                    // the same when the overflow may span several runs (syn_prime OVR)
+    float2* o; const float* w; int R; int ovd; int kov;    // outputs k < kov go to the overflow slot
+    SLICQ_DEVFN void st(int k, cpx v) const { cpx_st(o + R * k + (k < kov ? ovd : 0), cmulr(v, w[R * k])); }
 };
 struct PrimeDstAna {                       // analysis pass 1: output k1 -> stage[k1 * RP + n2] * twiddle
     float2* o; const float2* tw; int RP, R;
@@ -568,8 +583,8 @@ SLICQ_DEVFN void ana_prime(const SlicqBinsParams& p, const SlicqBucketArg& b, co
     }
 }
 
-// synthesis (prime last): x[P*n1 + n2], n1 in [0,R) -> X[k1 + R*k2], k2 in [0,P)
-template <int M, int P, int R>
+// synthesis (prime last): x[P*n1 + n2], n1 in [0,R) -> X[k1 + R*k2], k2 in [0,P); OVR as in syn_two_pass
+template <int M, int P, int R, bool OVR>
 SLICQ_DEVFN void syn_prime(const SlicqBinsParams& p, const SlicqBucketArg& b, const JobCtx& j, float* smf) {
     static_assert(P * R == M && R % 2 == 0, "bad split");
     constexpr int NP = (P <= 41 ? 2 : (P <= 61 ? 3 : 4));
@@ -636,6 +651,15 @@ SLICQ_DEVFN void syn_prime(const SlicqBinsParams& p, const SlicqBucketArg& b, co
             if (!(SLICQ_DBG_BINS & 4)) D::run(part, src, o);
             else { for (int q = 0; q < D::NOUT; ++q) o[q] = src.ld(q); }
             if ((SLICQ_DBG_BINS & 8) && p.n_rs >= 0) continue;
+            if (OVR) {   // outputs k1 + R k2 below the overflow count: k2 < ceil((count - k1) / R)
+                PrimeDstSynOvr dst;
+                dst.o = p.spec + SLICQ_TROW(base + gs) * p.spec_stride + tob[3 * f] + k1;
+                dst.w = wsm + f * M + k1; dst.R = R;
+                dst.ovd = tob[3 * f + 2] - tob[3 * f];
+                dst.kov = (tob[3 * f + 1] - k1 + R - 1) / R;
+                D::store(part, dst, o);
+                continue;
+            }
             PrimeDstSyn dst;
             dst.o = p.spec + SLICQ_TROW(base + gs) * p.spec_stride + tob[3 * f] + k1;
             dst.w = wsm + f * M + k1; dst.R = R;
