@@ -116,8 +116,7 @@ def profile_read(lib: C.CDLL | None = None) -> dict:
 
 
 def library_path() -> str:
-    # SLICQ_B200_LIB selects another *build of the same CUDA library* (kernel tuning sweeps)
-    return os.environ.get("SLICQ_B200_LIB") or os.path.join(_HERE, LIB_NAME)
+    return os.path.join(_HERE, LIB_NAME)
 
 
 _lib = None
@@ -137,8 +136,8 @@ def load(path: str | None = None) -> C.CDLL:
     if lib.slicq_abi_version() != 1:
         raise ImportError(f"{p}: ABI version {lib.slicq_abi_version()} != 1")
     if path is None:
-        # the product loader only takes CUDA builds: SLICQ_B200_LIB selects another build of the SAME library
-        # (tuning sweeps), never the host emulation of the test tier
+        # the product loader only takes CUDA builds: the host emulation library of the test tier (tests/emu) exports
+        # the same C ABI and must never stand in for the GPU
         if lib.slicq_build_kind() != 0:
             raise ImportError(f"{p} is not a CUDA build of libslicq (host emulation libraries are test infrastructure)")
         _lib = lib

@@ -12,12 +12,6 @@
 // per-launch job table) and owns a contiguous range of (row,slice) units of that bucket.
 #include "slicq_fft_tile.cuh"
 
-#if defined(SLICQ_PHASE_TIMING) && !defined(SLICQ_EMU)
-extern "C" int slicq_debug_set_bins_timing(long long* buf) { return (int)cudaMemcpyToSymbol(g_bins_phase_buf, &buf, sizeof buf); }
-#else
-extern "C" int slicq_debug_set_bins_timing(long long*) { return -1; }
-#endif
-
 namespace {
 
 SLICQ_DEVFN int find_bucket(const SlicqBinsParams& p, int job) {
@@ -93,40 +87,34 @@ SLICQ_DEVFN void bins_body(const SlicqBinsParams& p, unsigned char* smem) {
     }
 }
 
+// resident CTAs per SM the kernels are compiled for: caps a thread at 65536 / (3 * 256) = 85 registers
+constexpr int kBinsMinBlocks = 3;
+
 }  // namespace
 
-#ifndef SLICQ_BINS_THREADS
-#define SLICQ_BINS_THREADS 256
-#endif
-#ifndef SLICQ_BINS_MIN_BLOCKS
-#define SLICQ_BINS_MIN_BLOCKS (768 / SLICQ_BINS_THREADS)
-#endif
-
-__global__ void __launch_bounds__(SLICQ_BINS_THREADS, SLICQ_BINS_MIN_BLOCKS) bins_fwd_kernel(const __grid_constant__ SlicqBinsParams p) {
+__global__ void __launch_bounds__(kBinsThreads, kBinsMinBlocks) bins_fwd_kernel(const __grid_constant__ SlicqBinsParams p) {
     SLICQ_DYN_SMEM(unsigned char, smem);
     bins_body<false, false, false>(p, smem);
 }
 
 // the analysis with the mask-gradient epilogue (SlicqBinsParams::mask_grad): the adjoint-of-synthesis plan's
 // slicq_forward_mask_grad
-__global__ void __launch_bounds__(SLICQ_BINS_THREADS, SLICQ_BINS_MIN_BLOCKS) bins_fwd_mask_grad_kernel(const __grid_constant__ SlicqBinsParams p) {
+__global__ void __launch_bounds__(kBinsThreads, kBinsMinBlocks) bins_fwd_mask_grad_kernel(const __grid_constant__ SlicqBinsParams p) {
     SLICQ_DYN_SMEM(unsigned char, smem);
     bins_body<false, true, false>(p, smem);
 }
 
-__global__ void __launch_bounds__(SLICQ_BINS_THREADS, SLICQ_BINS_MIN_BLOCKS) bins_inv_kernel(const __grid_constant__ SlicqBinsParams p) {
+__global__ void __launch_bounds__(kBinsThreads, kBinsMinBlocks) bins_inv_kernel(const __grid_constant__ SlicqBinsParams p) {
     SLICQ_DYN_SMEM(unsigned char, smem);
     bins_body<true, false, false>(p, smem);
 }
 
 // the synthesis for plans whose two-pass or prime bins divert more than their first run of outputs to the overflow slot
 // (slicq_plan::ov_multi_run: the lowest bins of some Bark / mel filterbanks with few bins or a low fmin)
-__global__ void __launch_bounds__(SLICQ_BINS_THREADS, SLICQ_BINS_MIN_BLOCKS) bins_inv_ovr_kernel(const __grid_constant__ SlicqBinsParams p) {
+__global__ void __launch_bounds__(kBinsThreads, kBinsMinBlocks) bins_inv_ovr_kernel(const __grid_constant__ SlicqBinsParams p) {
     SLICQ_DYN_SMEM(unsigned char, smem);
     bins_body<true, false, true>(p, smem);
 }
-
-extern "C" int slicq_bins_threads(void) { return SLICQ_BINS_THREADS; }
 
 // host-side launcher (called from slicq_api.cu); synth: 0 analysis, 1 synthesis, 2 synthesis with overflow over several runs
 extern "C" int slicq_launch_bins(const SlicqBinsParams* p, int n_jobs, int smem_bytes, int synth, cudaStream_t s) {
@@ -146,13 +134,13 @@ extern "C" int slicq_launch_bins(const SlicqBinsParams* p, int n_jobs, int smem_
     }
 #endif
     if (synth == 2) {
-        SLICQ_LAUNCH(bins_inv_ovr_kernel, dim3(n_jobs), dim3(SLICQ_BINS_THREADS), smem_bytes, s, *p);
+        SLICQ_LAUNCH(bins_inv_ovr_kernel, dim3(n_jobs), dim3(kBinsThreads), smem_bytes, s, *p);
     } else if (synth) {
-        SLICQ_LAUNCH(bins_inv_kernel, dim3(n_jobs), dim3(SLICQ_BINS_THREADS), smem_bytes, s, *p);
+        SLICQ_LAUNCH(bins_inv_kernel, dim3(n_jobs), dim3(kBinsThreads), smem_bytes, s, *p);
     } else if (p->mask_grad) {
-        SLICQ_LAUNCH(bins_fwd_mask_grad_kernel, dim3(n_jobs), dim3(SLICQ_BINS_THREADS), smem_bytes, s, *p);
+        SLICQ_LAUNCH(bins_fwd_mask_grad_kernel, dim3(n_jobs), dim3(kBinsThreads), smem_bytes, s, *p);
     } else {
-        SLICQ_LAUNCH(bins_fwd_kernel, dim3(n_jobs), dim3(SLICQ_BINS_THREADS), smem_bytes, s, *p);
+        SLICQ_LAUNCH(bins_fwd_kernel, dim3(n_jobs), dim3(kBinsThreads), smem_bytes, s, *p);
     }
     return (int)cudaGetLastError();
 }

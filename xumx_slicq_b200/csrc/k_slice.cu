@@ -28,28 +28,15 @@
 #include "slicq_common.cuh"
 #include "dft_codelets.cuh"
 
-#ifndef SLICQ_SLICE_THREADS
-#define SLICQ_SLICE_THREADS 448
-#endif
-// tuning experiments only (results invalid): bit 0 skips the load phases of the synthesis slice kernel, bit 1 pass A,
-// bit 2 pass B, bit 3 the output stores
-// CTAs ahead whose input a CTA asks L2 to fetch while it transforms its own (0 = off).  Swept on the synthesis kernel:
+namespace {
+
+constexpr int kSliceThreads = 448;
+// CTAs ahead whose input a CTA asks L2 to fetch while it transforms its own (synthesis: kPrefetchAhead, analysis:
+// kPrefetchFwd).  Swept on the synthesis kernel:
 // 32 / 64 / 96 / 128 / 148 / 208 / 296 / 592 CTAs ahead = 0.520 / 0.505 / 0.506 / 0.511 / 0.512 / 0.521 / 0.545 / 0.620 ms (off: 0.545;
 // 296 CTAs are resident: further ahead the lines are evicted again before they are used)
-#ifndef SLICQ_PF_AHEAD
-#define SLICQ_PF_AHEAD 80
-#endif
-#ifndef SLICQ_PF_BULK
-#define SLICQ_PF_BULK 1
-#endif
-#ifndef SLICQ_PF_FWD
-#define SLICQ_PF_FWD 80
-#endif
-#ifndef SLICQ_DBG_SKIP
-#define SLICQ_DBG_SKIP 0
-#endif
-
-namespace {
+constexpr int kPrefetchAhead = 80;
+constexpr int kPrefetchFwd = 80;
 
 constexpr int cmodinv(int a, int m) {
     a %= m;
@@ -74,13 +61,9 @@ struct PfaNat {
     static constexpr int I2 = cmodinv(P3, P2), I3 = cmodinv(P2, P3);   // m -> (i2, i3) = (I2 m mod P2, I3 m mod P3)
     static_assert(C3 % P3 == 1, "orbit rotation of the last axis assumes (N / P3) mod P3 == 1");
     static_assert(SA >= P2 * SB && SB >= P3, "pitches too small");
-    static_assert(NP * SLOT <= SLICQ_SLICE_THREADS, "pass A needs NP * SLOT threads");
+    static_assert(NP * SLOT <= kSliceThreads, "pass A needs NP * SLOT threads");
 };
-#ifndef SLICQ_PFA_SB
-#define SLICQ_PFA_SB 16
-#define SLICQ_PFA_SA 243
-#endif
-typedef PfaNat<43, 15, 14, 2, SLICQ_PFA_SB, SLICQ_PFA_SA> Pfa9030;
+typedef PfaNat<43, 15, 14, 2, 16, 243> Pfa9030;
 
 // pass A sources / destinations (Dftp<>::run / store)
 template <class PF> struct ColNat {        // column m in natural order: element i1 at 43 m + 210 i1 (mod N)
@@ -117,7 +100,7 @@ SLICQ_DEVFN void pass_a(float2* Z) {
 // pass B: DFT-P2 along i2 for fixed (i1, i3), in place; lanes <-> i1 (pitch SA odd: conflict free)
 template <class PF, bool INV>
 SLICQ_DEVFN void pass_b(float2* Z) {
-    for (int t = threadIdx.x; t < PF::P1 * PF::P3; t += SLICQ_SLICE_THREADS) {
+    for (int t = threadIdx.x; t < PF::P1 * PF::P3; t += kSliceThreads) {
         const int i3 = t / PF::P1, i1 = t - i3 * PF::P1;
         float2* p = Z + i1 * PF::SA + i3;
         cpx v[PF::P2];
@@ -135,9 +118,9 @@ SLICQ_DEVFN void pass_b(float2* Z) {
 // ------------------------------------------------------------------------------------------
 // stage 1: one CTA per (row, slice).  x -> padded half spectrum H_ext[pad_l + f], f in [-pad_l, N + pad_r]
 template <class PF>
-__global__ void __launch_bounds__(SLICQ_SLICE_THREADS, 2) slice_fft_fwd_kernel(const __grid_constant__ SlicqSliceParams p) {
+__global__ void __launch_bounds__(kSliceThreads, 2) slice_fft_fwd_kernel(const __grid_constant__ SlicqSliceParams p) {
     SLICQ_DYN_SMEM(float2, Z);
-    constexpr int N = PF::N, NT = SLICQ_SLICE_THREADS, P3 = PF::P3, C3 = PF::C3;
+    constexpr int N = PF::N, NT = kSliceThreads, P3 = PF::P3, C3 = PF::C3;
     const int rsl = blockIdx.x;
     const int rs = p.rs0 + rsl;
     const int row = rs / p.S, k = rs - row * p.S;
@@ -147,17 +130,15 @@ __global__ void __launch_bounds__(SLICQ_SLICE_THREADS, 2) slice_fft_fwd_kernel(c
     const int e_lo = p.t.tw_lo >> 1, e_hi = (p.t.tw_hi + 1) >> 1;       // sample pairs with a non-zero window
     const long long sa = s0 + 2 * e_lo, sb = s0 + 2 * e_hi;             // x range touched by the window support
     const bool fast = sa >= 0 && sb <= p.T && ((reinterpret_cast<uintptr_t>(xr + s0) & 7) == 0);
-#if SLICQ_PF_FWD > 0
-    if (blockIdx.x + SLICQ_PF_FWD < gridDim.x) {
-        // the second half of the slice SLICQ_PF_FWD units ahead (its first half is the second half of its left neighbour)
-        const int rs2 = rs + SLICQ_PF_FWD;
+    if (blockIdx.x + kPrefetchFwd < gridDim.x) {
+        // the second half of the slice kPrefetchFwd units ahead (its first half is the second half of its left neighbour)
+        const int rs2 = rs + kPrefetchFwd;
         const int row2 = rs2 / p.S, k2 = rs2 - row2 * p.S;
         const long long a = (p.k0 + k2) * (long long)p.t.hop - p.t0;          // x index of the middle of that slice
         const float* __restrict__ x2r = p.x + row2 * p.x_row_stride;
         for (long long i = a + 32LL * threadIdx.x; i < a + p.t.hop; i += 32LL * NT)
             if (i >= 0 && i < p.T) prefetch_l2(x2r + i);
     }
-#endif
     // ---- windowed slice -> Z in natural order (coalesced loads; the zero part of the window is not read)
     if (fast) {
         const float2* __restrict__ x2 = reinterpret_cast<const float2*>(xr + s0);
@@ -268,9 +249,9 @@ __global__ void __launch_bounds__(SLICQ_SLICE_THREADS, 2) slice_fft_fwd_kernel(c
 // question arises) -- no intermediate slice buffer, and a two-term sum is order independent (bitwise reproducible).
 // (reference: nsgt/nsigtf.py:82-103, nsgt/unslicing.py:33-69, nsgt/slicq.py:207-230)
 template <class PF>
-__global__ void __launch_bounds__(SLICQ_SLICE_THREADS, 2) slice_fft_inv_kernel(const __grid_constant__ SlicqSliceParams p) {
+__global__ void __launch_bounds__(kSliceThreads, 2) slice_fft_inv_kernel(const __grid_constant__ SlicqSliceParams p) {
     SLICQ_DYN_SMEM(float2, Z);
-    constexpr int N = PF::N, NT = SLICQ_SLICE_THREADS, P3 = PF::P3, C3 = PF::C3;
+    constexpr int N = PF::N, NT = kSliceThreads, P3 = PF::P3, C3 = PF::C3;
     // CTA i of the launch = i-th slice of this launch's parity at or after unit rs0
     const int pi = p.par_base + blockIdx.x;
     const int row = pi / p.par_cs, k = 2 * (pi - row * p.par_cs) + p.parity;
@@ -282,7 +263,6 @@ __global__ void __launch_bounds__(SLICQ_SLICE_THREADS, 2) slice_fft_inv_kernel(c
     // pipe traffic); meanwhile every thread loads plane 1 at ITS pairs (k, N - k) into registers.  After the copy has
     // landed (mbarrier) and the overflow entries are added, a thread owns its pairs exclusively: it adds plane 1,
     // pre-processes and writes back in place.
-    if (!(SLICQ_DBG_SKIP & 1)) {
     constexpr int NP2 = (N / 2 + NT) / NT;      // pairs (k, N-k) per thread
     constexpr unsigned ROW_BYTES = (N / 2 + 1) * 16u;   // positions 0 .. N and one pad, rows are 16-byte aligned
 #ifdef SLICQ_EMU
@@ -312,20 +292,14 @@ __global__ void __launch_bounds__(SLICQ_SLICE_THREADS, 2) slice_fft_inv_kernel(c
         if (tid < p.t.n_ex) xe = __ldg(p.t.ex + tid);
         float2 x2 = make_float2(0.f, 0.f), x3 = make_float2(0.f, 0.f);
         if (xe.x >= 0) { x2 = __ldg(Trow + xe.y); if (xe.z >= 0) x3 = __ldg(Trow + xe.z); }
-#if SLICQ_PF_AHEAD > 0
         {   // while this CTA transforms, L2 fetches the row of the CTA that will run in this slot next (blockIdx + resident CTAs)
-            const int pj = pi + SLICQ_PF_AHEAD;
-            if (blockIdx.x + SLICQ_PF_AHEAD < gridDim.x) {
+            const int pj = pi + kPrefetchAhead;
+            if (blockIdx.x + kPrefetchAhead < gridDim.x) {
                 const int row2 = pj / p.par_cs, k2 = 2 * (pj - row2 * p.par_cs) + p.parity;
                 const float2* __restrict__ T2 = p.spec + (long long)(row2 * p.S + k2 - p.rs0) * p.spec_stride;
-#if SLICQ_PF_BULK
                 if (tid == 32) bulk_prefetch_l2(T2, (unsigned)p.t.t_stride * 8u);      // rows are 16-byte aligned, t_stride is even
-#else
-                for (int i = tid; 16 * i < p.t.t_stride; i += NT) prefetch_l2(T2 + 16 * i);
-#endif
             }
         }
-#endif
         mbar_wait(bar_, 0);
         // overflow entries: position f also receives T[off0] (+ T[off1]); entries have distinct f
         if (xe.x >= 0) { Z[xe.x].x += x2.x + x3.x; Z[xe.x].y += x2.y + x3.y; }
@@ -373,10 +347,9 @@ __global__ void __launch_bounds__(SLICQ_SLICE_THREADS, 2) slice_fft_inv_kernel(c
             }
         }
     }
-    }
     __syncthreads();
-    if (!(SLICQ_DBG_SKIP & 2)) pass_a<PF, true, ColNat<PF>, ColL2<PF> >(Z);
-    if (!(SLICQ_DBG_SKIP & 4)) pass_b<PF, true>(Z);
+    pass_a<PF, true, ColNat<PF>, ColL2<PF> >(Z);
+    pass_b<PF, true>(Z);
     // ---- pass C (last): thread t owns the orbit {t + C3 j} of the OUTPUT; element j has i3 = (t + j) mod P3.  The
     // outputs go back to Z in natural order (all tasks of a thread stay in registers until every thread has read its
     // inputs) and leave as 14 bulk copies / bulk reductions (one per row of C3 = 645 sample pairs, issued by lane 0 of
@@ -427,7 +400,6 @@ __global__ void __launch_bounds__(SLICQ_SLICE_THREADS, 2) slice_fft_inv_kernel(c
     float* __restrict__ halo = (p.halo_out != nullptr && p.k0 > 0) ? p.halo_out + (long long)row * p.t.hop : nullptr;
     const bool vec = ((reinterpret_cast<uintptr_t>(yr + tb) & 7) == 0) && tb >= 0 && tb + 2 * N <= p.T && !first_to_halo;
     const bool add1 = accumulate, add2 = accumulate && !second_store;
-    if (SLICQ_DBG_SKIP & 8) return;
     if (p.t.adjoint & 2) {
         // adjoint of the analysis: the slicing window multiplies the slice before the overlap-add
         __syncthreads();
@@ -500,7 +472,7 @@ extern "C" int slicq_launch_slice_fwd(const SlicqSliceParams* p, cudaStream_t s)
     if (p->t.L != 2 * Pfa9030::N) return slicq_launch_slice_fwd_generic(p, s);
     const int smem = (int)(Pfa9030::SMEM_ELEMS * sizeof(float2));
     if (slice_attr(smem)) return -3;
-    SLICQ_LAUNCH(slice_fft_fwd_kernel<Pfa9030>, dim3(p->n_rs), dim3(SLICQ_SLICE_THREADS), smem, s, *p);
+    SLICQ_LAUNCH(slice_fft_fwd_kernel<Pfa9030>, dim3(p->n_rs), dim3(kSliceThreads), smem, s, *p);
     return (int)cudaGetLastError();
 }
 
@@ -516,6 +488,6 @@ extern "C" int slicq_launch_slice_inv(const SlicqSliceParams* p, cudaStream_t s)
     if (c1 <= c0) return 0;
     SlicqSliceParams sp = *p;
     sp.par_cs = cs; sp.par_base = (int)c0;
-    SLICQ_LAUNCH(slice_fft_inv_kernel<Pfa9030>, dim3((unsigned)(c1 - c0)), dim3(SLICQ_SLICE_THREADS), smem, s, sp);
+    SLICQ_LAUNCH(slice_fft_inv_kernel<Pfa9030>, dim3((unsigned)(c1 - c0)), dim3(kSliceThreads), smem, s, sp);
     return (int)cudaGetLastError();
 }

@@ -59,7 +59,6 @@ extern "C" int slicq_launch_bins(const SlicqBinsParams* p, int n_tiles, int smem
 extern "C" int slicq_launch_slice_fwd(const SlicqSliceParams* p, cudaStream_t s);
 extern "C" int slicq_launch_slice_inv(const SlicqSliceParams* p, cudaStream_t s);
 extern "C" int slicq_slice_smem_bytes(int L);
-extern "C" int slicq_bins_threads(void);
 extern "C" int slicq_launch_mirror_fix(const SlicqBinsParams* p, cudaStream_t s);
 extern "C" int slicq_launch_mirror_adj(const SlicqBinsParams* p, cudaStream_t s);
 
@@ -146,7 +145,6 @@ template <class T> int upload(const std::vector<T>& h, const T** d, std::vector<
 
 }  // namespace
 
-#define SLICQ_MAX_WAYS 8
 struct slicq_plan {
     int L, N2, hop, J, sum_M;
     std::vector<int> bin_M, bin_pos, bin_coff;
@@ -159,16 +157,12 @@ struct slicq_plan {
     long long spec_stride_fwd;
     long long t_stride;   // complex elements per unit of the synthesis intermediate T
     long long chunk_bytes;
-    int target_jobs;      // CTAs per bins launch the job split aims for
-    int min_iters;        // ... but a job keeps at least this many iterations (instruction-cache reuse)
-    int only_bucket;      // -1, or (SLICQ_ONLY_BUCKET, tuning aid) the single bucket the bins kernels process
     // Large calls are split by rows into two halves that run on two internal streams (forked from and
     // joined back into the caller's stream): the memory-latency-bound and the issue-bound kernels of
     // the two halves overlap on the SMs.  Rows are independent, so the results do not change.
     long long split_units;          // split when the call has at least this many units (0 = never)
-    int split_ways;                 // row groups / internal streams of a split call (2 .. SLICQ_MAX_WAYS)
-    mutable cudaStream_t side[SLICQ_MAX_WAYS];
-    mutable cudaEvent_t ev_fork, ev_join[SLICQ_MAX_WAYS];
+    mutable cudaStream_t side[2];
+    mutable cudaEvent_t ev_fork, ev_join[2];
     mutable bool side_ready;
     // calls that split share the side streams and the fork / join events: their enqueue sequence (record, waits, launches,
     // joins) runs under this mutex, so that one thread's waits always see its own records.  Un-split calls take no lock.
@@ -206,7 +200,7 @@ extern "C" int slicq_profile_read(double* ms, int64_t* launches) {
 extern "C" void slicq_plan_destroy(slicq_plan* p) {
     if (!p) return;
     if (p->side_ready) {
-        for (int h = 0; h < SLICQ_MAX_WAYS; ++h) { cudaStreamDestroy(p->side[h]); cudaEventDestroy(p->ev_join[h]); }
+        for (int h = 0; h < 2; ++h) { cudaStreamDestroy(p->side[h]); cudaEventDestroy(p->ev_join[h]); }
         cudaEventDestroy(p->ev_fork);
     }
     for (void* q : p->owned) cudaFree(q);
@@ -278,12 +272,10 @@ extern "C" int slicq_plan_create(const slicq_tables* t, slicq_plan** out) {
     p->bins_smem = 0;
     for (Bucket& b : p->buckets) {
         const FftPlan* f = find_fft_plan(b.M);
-        const int nthr = slicq_bins_threads();
-        int gt = nthr / (b.n_bins * fft_threads_per_transform(*f));
+        int gt = kBinsThreads / (b.n_bins * fft_threads_per_transform(*f));
         if (gt < 1) gt = 1;
-        static const int stage_kb = getenv("SLICQ_BINS_STAGE_KB") ? atoi(getenv("SLICQ_BINS_STAGE_KB")) : 48;   // tuning aid
-        while (gt > 1 && b.n_bins * gt * b.smem_per_fft > stage_kb * 1024) --gt;
-        if (b.n_bins * fft_threads_per_transform(*f) > nthr) {
+        while (gt > 1 && b.n_bins * gt * b.smem_per_fft > 48 * 1024) --gt;
+        if (b.n_bins * fft_threads_per_transform(*f) > kBinsThreads) {
             delete p;
             return fail(SLICQ_E_UNSUPPORTED, "bucket has too many bins for one CTA");
         }
@@ -460,7 +452,7 @@ extern "C" int slicq_plan_create(const slicq_tables* t, slicq_plan** out) {
     }
     // (the adjoint-of-analysis plan has no such pass: the analysis reads the exact Hermitian mirror; the adjoint-of-synthesis
     // plan runs the pass's transpose, mirror_adj_kernel, after its analysis bins)
-    const int n_mir = (getenv("SLICQ_NO_MIRROR") || (t->flags & SLICQ_PLAN_ADJOINT_OF_ANALYSIS)) ? 0 : (int)mir.size();   // SLICQ_NO_MIRROR: verification aid (shows what the pass contributes)
+    const int n_mir = (t->flags & SLICQ_PLAN_ADJOINT_OF_ANALYSIS) ? 0 : (int)mir.size();
     if (mir.empty()) mir.push_back(SlicqMirrorEntry{0, 0.f});
     const int n_mir_bins = (int)mir_bins.size();
     if (mir_bins.empty()) mir_bins.push_back(SlicqMirrorBin{0, 0, 0, 0});
@@ -517,24 +509,9 @@ extern "C" int slicq_plan_create(const slicq_tables* t, slicq_plan** out) {
     long long mb = env ? atoll(env) : 2048;
     if (mb < 1) mb = 1;
     p->chunk_bytes = mb << 20;
-    const char* envj = getenv("SLICQ_BINS_JOBS");
-    // jobs per bins launch: 148 SMs x 3 resident CTAs x 10 waves for large launches (short jobs even out the tail;
-    // swept 666 ... 8880 at batch 8 in both rounds), 1184 for small ones (a job keeps enough iterations to amortise its
-    // set-up); SLICQ_BINS_JOBS fixes the number
-    p->target_jobs = envj ? atoi(envj) : 0;
-    if (p->target_jobs < 0) p->target_jobs = 0;
     const char* envs = getenv("SLICQ_SPLIT_UNITS");
     p->split_units = envs ? atoll(envs) : 1184;
-    const char* envw = getenv("SLICQ_SPLIT_WAYS");
-    p->split_ways = envw ? atoi(envw) : 2;
-    if (p->split_ways < 2) p->split_ways = 2;
-    if (p->split_ways > SLICQ_MAX_WAYS) p->split_ways = SLICQ_MAX_WAYS;
     p->side_ready = false;
-    const char* envb = getenv("SLICQ_ONLY_BUCKET");
-    p->only_bucket = envb ? atoi(envb) : -1;
-    const char* envi = getenv("SLICQ_BINS_MIN_ITERS");
-    p->min_iters = envi ? atoi(envi) : 1;
-    if (p->min_iters < 1) p->min_iters = 1;
     *out = p;
     return SLICQ_OK;
 }
@@ -584,9 +561,8 @@ namespace {
 bool use_split(const slicq_plan* p, int64_t n_rows, int64_t n_slices) {
     return p->split_units > 0 && n_rows >= 2 && n_rows * n_slices >= p->split_units;
 }
-// rows are dealt to `ways` groups of (almost) equal size; group h = rows [part_row0(h), part_row0(h + 1))
-int split_ways(const slicq_plan* p, int64_t n_rows) { return (int)(n_rows < p->split_ways ? n_rows : p->split_ways); }
-int64_t part_row0(int64_t n_rows, int ways, int h) { return n_rows * h / ways; }
+// a split call deals its rows to two groups of (almost) equal size; group h = rows [part_row0(h), part_row0(h + 1))
+int64_t part_row0(int64_t n_rows, int h) { return n_rows * h / 2; }
 size_t half_scratch(const slicq_plan* p, int64_t rows, int64_t n_slices, int inverse) {
     long long units = rows * n_slices;
     const long long c = chunk_units(p, inverse);
@@ -596,7 +572,7 @@ size_t half_scratch(const slicq_plan* p, int64_t rows, int64_t n_slices, int inv
 int ensure_side_streams(const slicq_plan* p) {
     if (p->side_ready) return 0;
     if (cudaEventCreateWithFlags(&p->ev_fork, cudaEventDisableTiming)) return -1;
-    for (int h = 0; h < SLICQ_MAX_WAYS; ++h)
+    for (int h = 0; h < 2; ++h)
         if (cudaStreamCreateWithFlags(&p->side[h], cudaStreamNonBlocking) || cudaEventCreateWithFlags(&p->ev_join[h], cudaEventDisableTiming))
             return -1;
     p->side_ready = true;
@@ -607,10 +583,9 @@ int ensure_side_streams(const slicq_plan* p) {
 extern "C" size_t slicq_scratch_bytes(const slicq_plan* p, int64_t n_rows, int64_t n_slices, int inverse) {
     if (!p || n_rows <= 0 || n_slices <= 0) return 0;
     if (use_split(p, n_rows, n_slices)) {
-        const int ways = split_ways(p, n_rows);
         size_t total = 256;
-        for (int h = 0; h < ways; ++h)
-            total += half_scratch(p, part_row0(n_rows, ways, h + 1) - part_row0(n_rows, ways, h), n_slices, inverse);
+        for (int h = 0; h < 2; ++h)
+            total += half_scratch(p, part_row0(n_rows, h + 1) - part_row0(n_rows, h), n_slices, inverse);
         return total;
     }
     return half_scratch(p, n_rows, n_slices, inverse) + 256;
@@ -623,7 +598,10 @@ int fill_bins_params(const slicq_plan* p, const slicq_bucket_view* views, SlicqB
     bp.n_buckets = (int)p->buckets.size();
     double total = 0.0;
     for (const Bucket& b : p->buckets) total += b.cost;
-    const int target = p->target_jobs > 0 ? p->target_jobs : std::min(4440, std::max(1184, 4 * n_rs));
+    // jobs per bins launch: 148 SMs x 3 resident CTAs x 10 waves for large launches (short jobs even out the tail;
+    // swept 666 ... 8880 at batch 8 in both rounds), 1184 for small ones (a job keeps enough iterations to amortise its
+    // set-up)
+    const int target = std::min(4440, std::max(1184, 4 * n_rs));
     for (size_t i = 0; i < p->buckets.size(); ++i) {
         const Bucket& b = p->buckets[i];
         SlicqBucketArg& a = bp.b[i];
@@ -635,13 +613,9 @@ int fill_bins_params(const slicq_plan* p, const slicq_bucket_view* views, SlicqB
         a.nptr = norms ? reinterpret_cast<float*>(norms[i].ptr) : nullptr;
         const slicq_bucket_view* aux = masks ? masks : norms;      // synthesis masks or analysis magnitudes: never both
         a.ms_row = aux ? aux[i].s_row : 0; a.ms_bin = aux ? aux[i].s_bin : 0; a.ms_slice = aux ? aux[i].s_slice : 0;
-        if (p->only_bucket >= 0 && (int)i != p->only_bucket) {       // tuning aid: time one bucket alone
-            a.units_per_job = b.gt; a.n_jobs = 0; a.job_start = jobs;
-            continue;
-        }
         const int groups = (n_rs + b.gt - 1) / b.gt;                 // iterations available in this chunk
         int nj = (int)(target * b.cost / total + 0.5);
-        if (nj > groups / p->min_iters) nj = groups / p->min_iters;
+        if (nj > groups) nj = groups;
         if (nj < 1) nj = 1;
         const int gpj = (groups + nj - 1) / nj;                      // iterations per job
         a.units_per_job = gpj * b.gt;
@@ -667,12 +641,11 @@ template <class F>
 int run_split(const slicq_plan* p, int64_t n_rows, int64_t n_slices, int inverse, void* scratch, cudaStream_t s, F fn) {
     std::lock_guard<std::mutex> lock(p->split_mutex);
     if (ensure_side_streams(p)) return fail(SLICQ_E_CUDA, "cannot create internal streams");
-    const int ways = split_ways(p, n_rows);
     unsigned char* base = reinterpret_cast<unsigned char*>(scratch);
     cudaEventRecord(p->ev_fork, s);
     int rc = 0;
-    for (int h = 0; h < ways && rc == 0; ++h) {
-        const int64_t r0 = part_row0(n_rows, ways, h), rows = part_row0(n_rows, ways, h + 1) - r0;
+    for (int h = 0; h < 2 && rc == 0; ++h) {
+        const int64_t r0 = part_row0(n_rows, h), rows = part_row0(n_rows, h + 1) - r0;
         cudaStreamWaitEvent(p->side[h], p->ev_fork, 0);
         rc = fn(r0, rows, base, p->side[h]);
         base += half_scratch(p, rows, n_slices, inverse);
@@ -700,11 +673,7 @@ int forward_impl(const slicq_plan* p, const float* x, int64_t n_rows, int64_t x_
         if (!buckets[i].ptr || (norms && !norms[i].ptr)) return fail(SLICQ_E_INVALID, "null bucket pointer");
     cudaStream_t s0 = reinterpret_cast<cudaStream_t>(stream);
     // mask gradient: output row r reads mixture row r % mix_rows, so a row group must start on a multiple of mix_rows
-    bool split = use_split(p, n_rows, n_slices);
-    if (split && mix_rows) {
-        const int ways = split_ways(p, n_rows);
-        for (int h = 1; h < ways; ++h) split = split && (part_row0(n_rows, ways, h) % mix_rows == 0);
-    }
+    const bool split = use_split(p, n_rows, n_slices) && (!mix_rows || part_row0(n_rows, 1) % mix_rows == 0);
     if (split) {
         return run_split(p, n_rows, n_slices, 0, scratch, s0, [&](int64_t r0, int64_t rows, void* scr, cudaStream_t st) {
             std::vector<slicq_bucket_view> v(buckets, buckets + p->buckets.size()), nv;
@@ -845,11 +814,7 @@ int inverse_impl(const slicq_plan* p, const slicq_bucket_view* buckets, const sl
         if (!buckets[i].ptr) return fail(SLICQ_E_INVALID, "null bucket pointer");
     cudaStream_t s0 = reinterpret_cast<cudaStream_t>(stream);
     // masked synthesis: output row r reads mixture row r % x_rows, so a row group must start on a multiple of x_rows
-    bool split = use_split(p, n_rows, n_slices);
-    if (split && masks) {
-        const int ways = split_ways(p, n_rows);
-        for (int h = 1; h < ways; ++h) split = split && (part_row0(n_rows, ways, h) % x_rows == 0);
-    }
+    const bool split = use_split(p, n_rows, n_slices) && (!masks || part_row0(n_rows, 1) % x_rows == 0);
     if (split) {
         return run_split(p, n_rows, n_slices, 1, scratch, s0, [&](int64_t r0, int64_t rows, void* scr, cudaStream_t st) {
             std::vector<slicq_bucket_view> v(buckets, buckets + p->buckets.size()), mv;
@@ -870,10 +835,8 @@ int inverse_one(const slicq_plan* p, const slicq_bucket_view* buckets, const sli
                 int64_t n_rows, int64_t n_slices, int64_t k0, float* y, int64_t y_row_stride, int64_t length,
                 int64_t t0, float* halo_out, void* scratch, cudaStream_t s) {
     const long long units = n_rows * n_slices, cu = chunk_units(p, 1);
-    const long long nu = units < cu ? units : cu;
     unsigned char* base = reinterpret_cast<unsigned char*>((reinterpret_cast<uintptr_t>(scratch) + 255) & ~(uintptr_t)255);
     float2* T = reinterpret_cast<float2*>(base);
-    (void)nu;
     SlicqBinsParams* bp = new SlicqBinsParams();
     bp->t = p->dev; bp->spec = T; bp->spec_stride = p->t_stride; bp->S = (int)n_slices;
     bp->x_rows = masks ? (int)x_rows : 0;

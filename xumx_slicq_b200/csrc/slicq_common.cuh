@@ -189,6 +189,8 @@ SLICQ_DEVFN void bulk_prefetch_l2(const void* p, unsigned bytes) {
 
 #define SLICQ_MAX_BUCKETS 96
 #define SLICQ_MAX_M 292
+// threads of a bins-kernel CTA (k_bins.cu); the plan sizes each bucket's units per iteration to fill them
+constexpr int kBinsThreads = 256;
 
 // ---------------------------------------------------------------------------------------
 // complex helpers

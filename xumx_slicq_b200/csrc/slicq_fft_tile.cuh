@@ -19,59 +19,11 @@
 #include "slicq_common.cuh"
 #include "dft_codelets.cuh"
 
-// optional tuning instrumentation (-DSLICQ_PHASE_TIMING): per-CTA accumulated cycles of the analysis
-// two-pass kernel's phases, written by thread 0 to a buffer registered with
-// slicq_debug_set_bins_timing() (tools/bins_timing.py).  Compiled out of the product build.
-#if defined(SLICQ_PHASE_TIMING) && !defined(SLICQ_EMU)
-__device__ long long* g_bins_phase_buf = nullptr;   // this header is included by k_bins.cu only
-#define BINS_T(v) const long long v = clock64()
-#define BINS_T0(v) long long v = 0
-#define BINS_SET(v) v = clock64()
-#define BINS_COUNT() do { if (threadIdx.x == 0) ++bins_iters_; } while (0)
-#define BINS_ACC(i, a, b) do { if (threadIdx.x == 0) bins_acc_[i] += (b) - (a); } while (0)
-#define BINS_DECL long long bins_acc_[6] = {0, 0, 0, 0, 0, 0}; long long bins_iters_ = 0
-#define BINS_FLUSH(M_) do { if (threadIdx.x == 0 && g_bins_phase_buf) { long long* o = g_bins_phase_buf + (long long)blockIdx.x * 8; \
-        for (int q_ = 0; q_ < 6; ++q_) o[q_] = bins_acc_[q_]; o[6] = (M_) | (bins_iters_ << 16); o[7] = 1; } } while (0)
-#else
-#define BINS_T(v) do {} while (0)
-#define BINS_T0(v) do {} while (0)
-#define BINS_SET(v) do {} while (0)
-#define BINS_COUNT() do {} while (0)
-#define BINS_ACC(i, a, b) do {} while (0)
-#define BINS_DECL do {} while (0)
-#define BINS_FLUSH(M_) do {} while (0)
-#endif
-
-// tuning experiment only (-DSLICQ_DEBUG_TWRAP=n): all units share n rows of the synthesis scratch, so that T
-// stays L2 resident (results are garbage; measures what an L2-resident intermediate would buy)
-#ifdef SLICQ_DEBUG_TWRAP
-#define SLICQ_TROW(u) ((long long)((u) % SLICQ_DEBUG_TWRAP))
-#else
-#define SLICQ_TROW(u) ((long long)(u))
-#endif
-// same idea for the caller's coefficients (-DSLICQ_DEBUG_CWRAP=n): the synthesis reads the first n units over and over
-#ifdef SLICQ_DEBUG_CWRAP
-#define SLICQ_CUNIT(u) ((u) % SLICQ_DEBUG_CWRAP)
-#else
-#define SLICQ_CUNIT(u) (u)
-#endif
-
 // independent 16-byte loads in flight per thread in the input loop of the single-thread synthesis transforms
-#ifndef SLICQ_UK1
-#define SLICQ_UK1 4
-#endif
+constexpr int kSynSingleLoads = 4;
 // two-pass synthesis transforms with A + B up to this bound prefetch their next inputs into registers (see syn_two_pass)
-// tuning experiments only (results invalid): bit 0 no coefficient loads, bit 1 no first-pass transform, bit 2 no second-pass
-// transform, bit 3 no stores to the plane rows (synthesis kernels)
-#ifndef SLICQ_DBG_BINS
-#define SLICQ_DBG_BINS 0
-#endif
-#ifndef SLICQ_K3_PAD
-#define SLICQ_K3_PAD 0
-#endif
-#ifndef SLICQ_PIPE_MAX
-#define SLICQ_PIPE_MAX 26
-#endif
+constexpr int kSynPipeMax = 26;
+
 struct JobCtx {
     int u0, u1;     // unit range of this job (indices local to the chunk)
     int F;          // bins in the bucket
@@ -94,7 +46,7 @@ SLICQ_DEVFN float2 cneg_if(float2 v, bool neg) { return neg ? make_float2(-v.x, 
 SLICQ_DEVFN void fill_slot_off(long long* so, const SlicqBucketArg& b, const JobCtx& j, int base, int ng, int x_rows) {
     for (int t = threadIdx.x; t < ng * j.F; t += blockDim.x) {
         const int gs = t / j.F, f = t - gs * j.F;
-        const int rs = SLICQ_CUNIT(j.rs0 + base + gs);
+        const int rs = j.rs0 + base + gs;
         const int row = rs / j.S, k = rs - row * j.S;
         const int rowx = x_rows ? row % x_rows : row;
         so[t] = rowx * b.s_row + f * b.s_bin + k * b.s_slice;
@@ -205,7 +157,7 @@ SLICQ_DEVFN void syn_single(const SlicqBinsParams& p, const SlicqBucketArg& b, c
         __syncthreads();
         if (vec) {
             // four independent 16-byte loads in flight per thread (a rolled loop would wait for each in turn)
-            constexpr int U = SLICQ_UK1;
+            constexpr int U = kSynSingleLoads;
             const int tot = ng * j.F * (M / 2);
             for (int t0 = tid; t0 < tot; t0 += U * blockDim.x) {
                 float4 v[U];
@@ -214,7 +166,7 @@ SLICQ_DEVFN void syn_single(const SlicqBinsParams& p, const SlicqBucketArg& b, c
                     const int t = t0 + u * blockDim.x;
                     if (t < tot) {
                         const int slot = t / (M / 2), n = 2 * (t - slot * (M / 2));
-                        v[u] = (SLICQ_DBG_BINS & 1) ? make_float4(1.f, 2.f, (float)n, 0.f) : *reinterpret_cast<const float4*>(b.ptr + so[slot] + n);
+                        v[u] = *reinterpret_cast<const float4*>(b.ptr + so[slot] + n);
                     }
                 }
 #pragma unroll
@@ -243,7 +195,7 @@ SLICQ_DEVFN void syn_single(const SlicqBinsParams& p, const SlicqBucketArg& b, c
             float2 v[M];
 #pragma unroll
             for (int n = 0; n < M; ++n) v[n] = cneg_if(stage[n], n & 1);
-            if (!(SLICQ_DBG_BINS & 6)) dft<M, false>(v);
+            dft<M, false>(v);
 #pragma unroll
             for (int m = 0; m < M; ++m) stage[m] = v[m];
         }
@@ -255,8 +207,7 @@ SLICQ_DEVFN void syn_single(const SlicqBinsParams& p, const SlicqBucketArg& b, c
             const float2* src = sm + (g * j.F + fb) * PITCH + n;
             const float w0 = wsm[e], w1 = wsm[e + 1];
             const int off = (n < tob[3 * fb + 1] ? tob[3 * fb + 2] : tob[3 * fb]) + n;
-            if ((SLICQ_DBG_BINS & 8) && p.n_rs >= 0) continue;
-            *reinterpret_cast<float4*>(p.spec + SLICQ_TROW(base + g) * p.spec_stride + off) =
+            *reinterpret_cast<float4*>(p.spec + (long long)(base + g) * p.spec_stride + off) =
                 make_float4(src[0].x * w0, src[0].y * w0, src[1].x * w1, src[1].y * w1);
         }
     }
@@ -296,9 +247,7 @@ SLICQ_DEVFN void ana_two_pass(const SlicqBinsParams& p, const SlicqBucketArg& b,
     }
     const float2* twp = twsm + n2;
     __syncthreads();
-    BINS_DECL;
     for (int base = j.u0; base < j.u1; base += j.gt) {
-        BINS_T(t0_);
         const int g = base + gs1;
         const int ng = (j.u1 - base < j.gt) ? (j.u1 - base) : j.gt;
         fill_slot_off(so, b, j, base, ng, MG ? p.x_rows : 0);
@@ -316,9 +265,7 @@ SLICQ_DEVFN void ana_two_pass(const SlicqBinsParams& p, const SlicqBucketArg& b,
             for (int k1 = 1; k1 < A; ++k1)
                 y1[k1 * BP] = cneg_if(cmul_conj(v[k1], twp[k1 * B]), k1 & 1);  // (-1)^k1 folded here
         }
-        BINS_T(t1_);
         __syncthreads();
-        BINS_T(t2_);
         for (int t = tid; t < ng * j.F * A; t += blockDim.x) {
             const int slot = t / A, k1 = t - slot * A;
             const float2* src = sm + slot * PER + k1 * BP;
@@ -341,12 +288,8 @@ SLICQ_DEVFN void ana_two_pass(const SlicqBinsParams& p, const SlicqBucketArg& b,
                 for (int k2 = 0; k2 < B; ++k2) on[A * k2] = cmag(v[k2]);
             }
         }
-        BINS_T(t3_);
         __syncthreads();
-        BINS_T(t4_);
-        BINS_ACC(1, t0_, t1_); BINS_ACC(2, t1_, t2_); BINS_ACC(3, t2_, t3_); BINS_ACC(4, t3_, t4_); BINS_ACC(5, t0_, t4_);
     }
-    BINS_FLUSH(M);
 }
 
 // synthesis: x[B*n1 + n2] -> X[k1 + A*k2];  same shape as the analysis: pass 1 = DFT-A with the
@@ -388,28 +331,25 @@ SLICQ_DEVFN void syn_two_pass(const SlicqBinsParams& p, const SlicqBucketArg& b,
     }
     const float2* twp = twsm + n2;
     __syncthreads();
-    BINS_DECL;
-    // Software pipeline (sizes whose two register sets fit, A + B <= SLICQ_PIPE_MAX): the inputs of the NEXT group of units are
+    // Software pipeline (sizes whose two register sets fit, A + B <= kSynPipeMax): the inputs of the NEXT group of units are
     // requested right after pass 1 has put its outputs into shared memory, so that they travel during the barrier and pass 2.
-    constexpr bool PIPE = (A + B <= SLICQ_PIPE_MAX);
+    constexpr bool PIPE = (A + B <= kSynPipeMax);
     float2 v[A];
     int rowk[2] = {0, 0};           // (row, slice) of the unit whose inputs sit in v
     auto request = [&](int base) {
         const int g = base + gs1;
         if (act1 && g < j.u1) {
-            const int rs = SLICQ_CUNIT(j.rs0 + g);
+            const int rs = j.rs0 + g;
             const int row = rs / j.S, k = rs - row * j.S;
             const int rowx = j.x_rows ? row % j.x_rows : row;
             const float2* src = b.ptr + rowx * b.s_row + f1 * b.s_bin + k * b.s_slice + n2;
 #pragma unroll
-            for (int n1 = 0; n1 < A; ++n1) v[n1] = (SLICQ_DBG_BINS & 1) ? make_float2((float)n1, (float)k) : src[B * n1];
+            for (int n1 = 0; n1 < A; ++n1) v[n1] = src[B * n1];
             rowk[0] = row; rowk[1] = k;
         }
     };
     if (PIPE) request(j.u0);
     for (int base = j.u0; base < j.u1; base += j.gt) {
-        BINS_T(t0_);
-        BINS_T0(tl_);
         const int g = base + gs1;
         if (!PIPE) request(base);
         if (act1 && g < j.u1) {
@@ -420,16 +360,13 @@ SLICQ_DEVFN void syn_two_pass(const SlicqBinsParams& p, const SlicqBucketArg& b,
 #pragma unroll
                 for (int n1 = 0; n1 < A; ++n1) v[n1] = cscale(v[n1], msrc[B * n1]);
             }
-            BINS_SET(tl_);
-            if (!(SLICQ_DBG_BINS & 2)) dft<A, false>(v);
+            dft<A, false>(v);
             y1[0] = v[0];
 #pragma unroll
             for (int k1 = 1; k1 < A; ++k1) y1[k1 * BP] = cmul(v[k1], twp[k1 * B]);
         }
         if (PIPE && base + j.gt < j.u1) request(base + j.gt);
-        BINS_T(t1_);
         __syncthreads();
-        BINS_T(t2_);
         const int ng = (j.u1 - base < j.gt) ? (j.u1 - base) : j.gt;
         for (int t = tid; t < ng * j.F * A; t += blockDim.x) {
             const int slot = t / A, k1 = t - slot * A;
@@ -438,18 +375,10 @@ SLICQ_DEVFN void syn_two_pass(const SlicqBinsParams& p, const SlicqBucketArg& b,
             float2 v[B];
 #pragma unroll
             for (int n = 0; n < B; ++n) v[n] = src[n];
-            if (!(SLICQ_DBG_BINS & 4)) dft<B, false>(v);
-            if ((SLICQ_DBG_BINS & 8) && p.n_rs >= 0) continue;
-            float2* row = p.spec + SLICQ_TROW(base + (c.x & 0xffff)) * p.spec_stride;
+            dft<B, false>(v);
+            float2* row = p.spec + (long long)(base + (c.x & 0xffff)) * p.spec_stride;
             float2* o = row + c.y + k1;
             const float* wp = wsm + (c.x >> 16) * M + k1;
-            if (SLICQ_DBG_BINS & 16) {   // probe: the same bytes as fully coalesced stores (garbage layout)
-                float2* oc = p.spec + SLICQ_TROW(base) * p.spec_stride + t;
-                const int nt = ng * j.F * A;
-#pragma unroll
-                for (int k2 = 0; k2 < B; ++k2) oc[k2 * nt] = make_float2(v[k2].x * wp[A * k2], v[k2].y * wp[A * k2]);
-                continue;
-            }
             if (OVR) {   // any output k1 + A k2 below the overflow count goes to the overflow slot
 #pragma unroll
                 for (int k2 = 0; k2 < B; ++k2) {
@@ -471,13 +400,8 @@ SLICQ_DEVFN void syn_two_pass(const SlicqBinsParams& p, const SlicqBucketArg& b,
                 o[A * k2] = make_float2(v[k2].x * w, v[k2].y * w);
             }
         }
-        BINS_T(t3_);
         __syncthreads();
-        BINS_T(t4_);
-        BINS_ACC(0, t0_, tl_); BINS_ACC(1, tl_, t1_); BINS_ACC(2, t1_, t2_); BINS_ACC(3, t2_, t3_); BINS_ACC(4, t3_, t4_); BINS_ACC(5, t0_, t4_);
-        BINS_COUNT();
     }
-    BINS_FLUSH(M);
 }
 
 // =========================================================================================
@@ -595,7 +519,6 @@ SLICQ_DEVFN void syn_prime(const SlicqBinsParams& p, const SlicqBucketArg& b, co
     // job twiddles [k1][n2] = exp(-2 pi i n2 k1 / M) (-1)^n2, the bucket's dual windows and the T-row offsets of its bins
     // slot pitch M: pass 2 then reads column k1 of slot s at (s R + k1) P + n -- a single odd stride across the lanes
     // (a pitch of M + P put every half warp on 8 bank pairs: 2-way conflicts on the NP-times repeated loads of pass 2)
-    constexpr int SP = M + SLICQ_K3_PAD * P;
     float2* twsm = sm + (size_t)j.gt * j.F * (M + P);
     float* wsm = reinterpret_cast<float*>(twsm + M);
     const int coff_first = __ldg(p.t.bin_coff + j.first_bin);
@@ -626,14 +549,14 @@ SLICQ_DEVFN void syn_prime(const SlicqBinsParams& p, const SlicqBucketArg& b, co
             const float2* src = b.ptr + so[s] + c2;
             cpx v[R];
 #pragma unroll
-            for (int n1 = 0; n1 < R; ++n1) v[n1] = (SLICQ_DBG_BINS & 1) ? cpx_make((float)n1, (float)c2) : cpx_ld(src + P * n1);
+            for (int n1 = 0; n1 < R; ++n1) v[n1] = cpx_ld(src + P * n1);
             if (b.mptr != nullptr) {
                 const float* msrc = b.mptr + so[256 + s] + c2;
 #pragma unroll
                 for (int n1 = 0; n1 < R; ++n1) v[n1] = cmulr(v[n1], msrc[P * n1]);
             }
-            if (!(SLICQ_DBG_BINS & 2)) dft<R, false>(v);
-            float2* o = sm + s * SP + c2;
+            dft<R, false>(v);
+            float2* o = sm + s * M + c2;
             const float2* twp = twsm + c2;
 #pragma unroll
             for (int k1 = 0; k1 < R; ++k1) cpx_st(o + k1 * P, cmulw(v[(k1 + R / 2) % R], twp[k1 * P]));
@@ -646,14 +569,12 @@ SLICQ_DEVFN void syn_prime(const SlicqBinsParams& p, const SlicqBucketArg& b, co
             if (c >= ncol) continue;
             const int s = c / R, k1 = c - s * R;
             const int gs = s / j.F, f = s - gs * j.F;
-            PrimeSrcSyn<M> src; src.p = sm + s * SP + k1 * P;
+            PrimeSrcSyn<M> src; src.p = sm + s * M + k1 * P;
             cpx o[D::NOUT];
-            if (!(SLICQ_DBG_BINS & 4)) D::run(part, src, o);
-            else { for (int q = 0; q < D::NOUT; ++q) o[q] = src.ld(q); }
-            if ((SLICQ_DBG_BINS & 8) && p.n_rs >= 0) continue;
+            D::run(part, src, o);
             if (OVR) {   // outputs k1 + R k2 below the overflow count: k2 < ceil((count - k1) / R)
                 PrimeDstSynOvr dst;
-                dst.o = p.spec + SLICQ_TROW(base + gs) * p.spec_stride + tob[3 * f] + k1;
+                dst.o = p.spec + (long long)(base + gs) * p.spec_stride + tob[3 * f] + k1;
                 dst.w = wsm + f * M + k1; dst.R = R;
                 dst.ovd = tob[3 * f + 2] - tob[3 * f];
                 dst.kov = (tob[3 * f + 1] - k1 + R - 1) / R;
@@ -661,7 +582,7 @@ SLICQ_DEVFN void syn_prime(const SlicqBinsParams& p, const SlicqBucketArg& b, co
                 continue;
             }
             PrimeDstSyn dst;
-            dst.o = p.spec + SLICQ_TROW(base + gs) * p.spec_stride + tob[3 * f] + k1;
+            dst.o = p.spec + (long long)(base + gs) * p.spec_stride + tob[3 * f] + k1;
             dst.w = wsm + f * M + k1; dst.R = R;
             dst.ovd = (k1 < tob[3 * f + 1]) ? tob[3 * f + 2] - tob[3 * f] : 0;
             D::store(part, dst, o);
