@@ -116,31 +116,22 @@ __global__ void __launch_bounds__(kBinsThreads, kBinsMinBlocks) bins_inv_ovr_ker
     bins_body<true, false, true>(p, smem);
 }
 
-// host-side launcher (called from slicq_api.cu); synth: 0 analysis, 1 synthesis, 2 synthesis with overflow over several runs
-extern "C" int slicq_launch_bins(const SlicqBinsParams* p, int n_jobs, int smem_bytes, int synth, cudaStream_t s) {
-    if (n_jobs <= 0) return 0;
-#ifndef SLICQ_EMU
-    {   // cudaFuncSetAttribute is per device
-        static bool done[64] = {false};
-        int dev = 0;
-        if (cudaGetDevice(&dev) != cudaSuccess) return -3;
-        if (dev < 0 || dev >= 64 || !done[dev]) {
-            if (SLICQ_SET_SMEM(bins_fwd_kernel, 100 * 1024) != cudaSuccess) return -3;
-            if (SLICQ_SET_SMEM(bins_inv_kernel, 100 * 1024) != cudaSuccess) return -3;
-            if (SLICQ_SET_SMEM(bins_fwd_mask_grad_kernel, 100 * 1024) != cudaSuccess) return -3;
-            if (SLICQ_SET_SMEM(bins_inv_ovr_kernel, 100 * 1024) != cudaSuccess) return -3;
-            if (dev >= 0 && dev < 64) done[dev] = true;
-        }
-    }
-#endif
-    if (synth == 2) {
-        SLICQ_LAUNCH(bins_inv_ovr_kernel, dim3(n_jobs), dim3(kBinsThreads), smem_bytes, s, *p);
-    } else if (synth) {
-        SLICQ_LAUNCH(bins_inv_kernel, dim3(n_jobs), dim3(kBinsThreads), smem_bytes, s, *p);
-    } else if (p->mask_grad) {
-        SLICQ_LAUNCH(bins_fwd_mask_grad_kernel, dim3(n_jobs), dim3(kBinsThreads), smem_bytes, s, *p);
-    } else {
-        SLICQ_LAUNCH(bins_fwd_kernel, dim3(n_jobs), dim3(kBinsThreads), smem_bytes, s, *p);
-    }
+namespace {
+template <auto K> int launch_bins(const SlicqBinsParams* p, int n_jobs, int smem_bytes, cudaStream_t s) {
+    if (slicq_smem_opt_in<K>(100 * 1024)) return -3;
+    SLICQ_LAUNCH(K, dim3(n_jobs), dim3(kBinsThreads), smem_bytes, s, *p);
     return (int)cudaGetLastError();
+}
+}  // namespace
+
+// host-side launcher (called from slicq_api.cu)
+extern "C" int slicq_launch_bins(const SlicqBinsParams* p, int n_jobs, int smem_bytes, SlicqBinsKernel k, cudaStream_t s) {
+    if (n_jobs <= 0) return 0;
+    switch (k) {
+        case bins_fwd: return launch_bins<bins_fwd_kernel>(p, n_jobs, smem_bytes, s);
+        case bins_fwd_mask_grad: return launch_bins<bins_fwd_mask_grad_kernel>(p, n_jobs, smem_bytes, s);
+        case bins_inv: return launch_bins<bins_inv_kernel>(p, n_jobs, smem_bytes, s);
+        case bins_inv_ovr: return launch_bins<bins_inv_ovr_kernel>(p, n_jobs, smem_bytes, s);
+    }
+    return -2;
 }

@@ -453,25 +453,11 @@ extern "C" int slicq_slice_smem_bytes(int L) {
     return slicq_generic_smem_bytes(L);
 }
 
-// cudaFuncSetAttribute is per device: remember which devices have the opt-in for > 48 KB dynamic shared memory
-static int slice_attr(int smem) {
-#ifndef SLICQ_EMU
-    static bool done[64] = {false};
-    int dev = 0;
-    if (cudaGetDevice(&dev) != cudaSuccess) return -1;
-    if (dev >= 0 && dev < 64 && done[dev]) return 0;
-    if (SLICQ_SET_SMEM(slice_fft_fwd_kernel<Pfa9030>, smem) != cudaSuccess) return -1;
-    if (SLICQ_SET_SMEM(slice_fft_inv_kernel<Pfa9030>, smem) != cudaSuccess) return -1;
-    if (dev >= 0 && dev < 64) done[dev] = true;
-#endif
-    return 0;
-}
-
 extern "C" int slicq_launch_slice_fwd(const SlicqSliceParams* p, cudaStream_t s) {
     if (p->n_rs <= 0) return 0;
     if (p->t.L != 2 * Pfa9030::N) return slicq_launch_slice_fwd_generic(p, s);
     const int smem = (int)(Pfa9030::SMEM_ELEMS * sizeof(float2));
-    if (slice_attr(smem)) return -3;
+    if (slicq_smem_opt_in<slice_fft_fwd_kernel<Pfa9030>>(smem)) return -3;
     SLICQ_LAUNCH(slice_fft_fwd_kernel<Pfa9030>, dim3(p->n_rs), dim3(kSliceThreads), smem, s, *p);
     return (int)cudaGetLastError();
 }
@@ -480,14 +466,10 @@ extern "C" int slicq_launch_slice_inv(const SlicqSliceParams* p, cudaStream_t s)
     if (p->n_rs <= 0) return 0;
     if (p->t.L != 2 * Pfa9030::N) return slicq_launch_slice_inv_generic(p, s);
     const int smem = (int)(Pfa9030::SMEM_ELEMS * sizeof(float2));
-    if (slice_attr(smem)) return -3;
-    // slices of parity q among units [0, u) of rows of S slices
-    const int S = p->S, q = p->parity, cs = (S + 1 - q) / 2;
-    auto count = [&](long long u) { return (u / S) * cs + ((u % S) + 1 - q) / 2; };
-    const long long c0 = count(p->rs0), c1 = count((long long)p->rs0 + p->n_rs);
-    if (c1 <= c0) return 0;
-    SlicqSliceParams sp = *p;
-    sp.par_cs = cs; sp.par_base = (int)c0;
-    SLICQ_LAUNCH(slice_fft_inv_kernel<Pfa9030>, dim3((unsigned)(c1 - c0)), dim3(kSliceThreads), smem, s, sp);
+    if (slicq_smem_opt_in<slice_fft_inv_kernel<Pfa9030>>(smem)) return -3;
+    SlicqSliceParams sp;
+    const unsigned ctas = slicq_parity_ctas(*p, sp);
+    if (!ctas) return 0;
+    SLICQ_LAUNCH(slice_fft_inv_kernel<Pfa9030>, dim3(ctas), dim3(kSliceThreads), smem, s, sp);
     return (int)cudaGetLastError();
 }

@@ -300,24 +300,11 @@ extern "C" int slicq_generic_smem_bytes(int L) {
     return (L > 0 && L % 4 == 0 && b <= 220 * 1024) ? (int)b : -1;
 }
 
-static int generic_attr(int smem) {
-#ifndef SLICQ_EMU
-    static int done[64] = {0};
-    int dev = 0;
-    if (cudaGetDevice(&dev) != cudaSuccess) return -1;
-    if (dev >= 0 && dev < 64 && done[dev] >= smem) return 0;
-    if (SLICQ_SET_SMEM(slice_fft_fwd_generic_kernel, smem) != cudaSuccess) return -1;
-    if (SLICQ_SET_SMEM(slice_fft_inv_generic_kernel, smem) != cudaSuccess) return -1;
-    if (dev >= 0 && dev < 64) done[dev] = smem;
-#endif
-    return 0;
-}
-
 extern "C" int slicq_launch_slice_fwd_generic(const SlicqSliceParams* p, cudaStream_t s) {
     if (p->n_rs <= 0) return 0;
     const int smem = slicq_generic_smem_bytes(p->t.L);
     if (smem < 0) return -2;
-    if (generic_attr(smem)) return -3;
+    if (slicq_smem_opt_in<slice_fft_fwd_generic_kernel>(smem)) return -3;
     SLICQ_LAUNCH(slice_fft_fwd_generic_kernel, dim3(p->n_rs), dim3(SLICQ_GEN_THREADS), smem, s, *p);
     return (int)cudaGetLastError();
 }
@@ -326,14 +313,11 @@ extern "C" int slicq_launch_slice_inv_generic(const SlicqSliceParams* p, cudaStr
     if (p->n_rs <= 0) return 0;
     const int smem = slicq_generic_smem_bytes(p->t.L);
     if (smem < 0) return -2;
-    if (generic_attr(smem)) return -3;
-    const int S = p->S, q = p->parity, cs = (S + 1 - q) / 2;
-    auto count = [&](long long u) { return (u / S) * cs + ((u % S) + 1 - q) / 2; };
-    const long long c0 = count(p->rs0), c1 = count((long long)p->rs0 + p->n_rs);
-    if (c1 <= c0) return 0;
-    SlicqSliceParams sp = *p;
-    sp.par_cs = cs; sp.par_base = (int)c0;
-    SLICQ_LAUNCH(slice_fft_inv_generic_kernel, dim3((unsigned)(c1 - c0)), dim3(SLICQ_GEN_THREADS), smem, s, sp);
+    if (slicq_smem_opt_in<slice_fft_inv_generic_kernel>(smem)) return -3;
+    SlicqSliceParams sp;
+    const unsigned ctas = slicq_parity_ctas(*p, sp);
+    if (!ctas) return 0;
+    SLICQ_LAUNCH(slice_fft_inv_generic_kernel, dim3(ctas), dim3(SLICQ_GEN_THREADS), smem, s, sp);
     return (int)cudaGetLastError();
 }
 

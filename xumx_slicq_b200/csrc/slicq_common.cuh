@@ -320,3 +320,41 @@ struct SlicqSliceParams {
     int parity;            // inverse: this launch handles slices with (k & 1) == parity ...
     int par_cs, par_base;  // ... one CTA each: par_cs = such slices per row, par_base = how many precede unit rs0 (set by the launcher)
 };
+
+// ---------------------------------------------------------------------------------------
+// host-side launcher helpers (k_bins.cu, k_slice.cu, k_slice_generic.cu)
+#include <atomic>
+#include <mutex>
+
+// the four variants of the bins kernel (k_bins.cu)
+enum SlicqBinsKernel { bins_fwd, bins_fwd_mask_grad, bins_inv, bins_inv_ovr };
+
+// Opts kernel K in to `bytes` of dynamic shared memory on the current device (the attribute is per device).  The largest
+// value set so far is recorded per device; a call that needs no more returns at once, the others set the attribute under
+// a lock, so that the attribute only ever rises, also when threads of plans of different lengths race.  0 on success.
+template <auto K>
+static int slicq_smem_opt_in(int bytes) {
+    static std::atomic<int> done[64];
+    static std::mutex m;
+    int dev = 0;
+    if (cudaGetDevice(&dev) != cudaSuccess) return -1;
+    std::atomic<int>* rec = (dev >= 0 && dev < 64) ? &done[dev] : nullptr;   // devices beyond the 64th: set every time
+    if (rec && rec->load(std::memory_order_acquire) >= bytes) return 0;
+    std::lock_guard<std::mutex> lock(m);
+    if (rec && rec->load(std::memory_order_relaxed) >= bytes) return 0;
+    if (SLICQ_SET_SMEM(K, bytes) != cudaSuccess) return -1;
+    if (rec) rec->store(bytes, std::memory_order_release);
+    return 0;
+}
+
+// The inverse slice kernels run one launch per slice parity, one CTA per slice k with (k & 1) == p.parity among the
+// units [rs0, rs0 + n_rs) of rows of S slices.  Sets par_cs (such slices per row) and par_base (how many precede unit rs0)
+// in `sp` (a copy of p) and returns the number of CTAs, 0 if there are none.
+static inline unsigned slicq_parity_ctas(const SlicqSliceParams& p, SlicqSliceParams& sp) {
+    const int S = p.S, q = p.parity, cs = (S + 1 - q) / 2;
+    auto count = [&](long long u) { return (u / S) * cs + ((u % S) + 1 - q) / 2; };
+    const long long c0 = count(p.rs0), c1 = count((long long)p.rs0 + p.n_rs);
+    sp = p;
+    sp.par_cs = cs; sp.par_base = (int)c0;
+    return c1 > c0 ? (unsigned)(c1 - c0) : 0u;
+}
