@@ -5,7 +5,8 @@
 // (one output per thread and stage: O(N sum p) operations, any factor, natural order in and out; twiddles from one table
 // exp(-2 pi i k / N)).  Correct for every N that fits two buffers in shared memory, not tuned: the roofline work is the
 // pretrained configuration's.  Also here: the reference's mirrored-bin pass (nsgt/nsigtf.py:63-80) for configurations
-// where a bin reaches below DC, so that its mirror image wraps into the kept half spectrum, and its transpose.
+// where a bin reaches below DC, so that its mirror image wraps into the kept half spectrum, and its transpose; and the
+// transforms of the long Nyquist bin of band-limited filterbanks (fmax < fs / 2) on the same Stockham engine.
 #include "slicq_common.cuh"
 
 #define SLICQ_GEN_THREADS 256
@@ -14,13 +15,13 @@ namespace {
 
 SLICQ_DEVFN float2 gmul(float2 a, float2 b) { return make_float2(fmaf(a.x, b.x, -a.y * b.y), fmaf(a.x, b.y, a.y * b.x)); }
 
-// x -> FFT (sign -) or unnormalised inverse FFT (sign +) of length N; returns the buffer that holds the result
+// x -> FFT (sign -) or unnormalised inverse FFT (sign +) of length N = prod fac[0 .. n_fac) (largest factor first);
+// wN = exp(-2 pi i k / N), wP = exp(-2 pi i k / fac[0]) in double when fac[0] > 32.  Returns the buffer that holds the result
 template <bool INV>
-SLICQ_DEVFN float2* stockham(float2* x, float2* y, const SlicqDeviceTables& t) {
-    const int N = t.N2;
+SLICQ_DEVFN float2* stockham(float2* x, float2* y, int N, int n_fac, const int* fac, const float2* wN, const double2* wP) {
     int n = N, s = 1;
-    for (int st = 0; st < t.n_fac; ++st) {
-        const int pf = t.fac[st], m = n / pf;
+    for (int st = 0; st < n_fac; ++st) {
+        const int pf = fac[st], m = n / pf;
         const int wp = N / pf, wn = N / n;
         for (int idx = threadIdx.x; idx < N; idx += SLICQ_GEN_THREADS) {
             // output idx = r + s (pf q + j)  <-  inputs r + s (q + m k), k < pf
@@ -32,7 +33,7 @@ SLICQ_DEVFN float2* stockham(float2* x, float2* y, const SlicqDeviceTables& t) {
             if (pf <= 32 || st != 0) {       // only the largest factor (first stage) has a double table
                 for (int k = 1; k < pf; ++k) {
                     jk += j; if (jk >= pf) jk -= pf;
-                    float2 w = __ldg(t.wN + wp * jk);
+                    float2 w = __ldg(wN + wp * jk);
                     if (INV) w.y = -w.y;
                     const float2 a = src[s * m * k];
                     acc.x += a.x * w.x - a.y * w.y;
@@ -45,7 +46,7 @@ SLICQ_DEVFN float2* stockham(float2* x, float2* y, const SlicqDeviceTables& t) {
                 double ax = acc.x, ay = acc.y;
                 for (int k = 1; k < pf; ++k) {
                     jk += j; if (jk >= pf) jk -= pf;
-                    double2 w = t.wP[jk];
+                    double2 w = wP[jk];
                     if (INV) w.y = -w.y;
                     const float2 a = src[s * m * k];
                     ax += (double)a.x * w.x - (double)a.y * w.y;
@@ -53,7 +54,7 @@ SLICQ_DEVFN float2* stockham(float2* x, float2* y, const SlicqDeviceTables& t) {
                 }
                 acc = make_float2((float)ax, (float)ay);
             }
-            float2 tw = __ldg(t.wN + wn * j * q);
+            float2 tw = __ldg(wN + wn * j * q);
             if (INV) tw.y = -tw.y;
             y[idx] = gmul(acc, tw);
         }
@@ -85,7 +86,7 @@ __global__ void __launch_bounds__(SLICQ_GEN_THREADS, 1) slice_fft_fwd_generic_ke
         A[e] = make_float2(a, b);
     }
     __syncthreads();
-    const float2* Z = stockham<false>(A, B, p.t);
+    const float2* Z = stockham<false>(A, B, N, p.t.n_fac, p.t.fac, p.t.wN, p.t.wP);
     float2* __restrict__ H = p.spec + (long long)rsl * p.spec_stride + p.t.pad_l;
     const int pad_l = p.t.pad_l, pad_r = p.t.pad_r;
     const float sc = p.t.spec_scale, se = p.t.ends_scale;
@@ -178,7 +179,7 @@ __global__ void __launch_bounds__(SLICQ_GEN_THREADS, 1) slice_fft_inv_generic_ke
         }
     }
     __syncthreads();
-    const float2* Z = stockham<true>(A, B, p.t);
+    const float2* Z = stockham<true>(A, B, N, p.t.n_fac, p.t.fac, p.t.wN, p.t.wP);
     const long long tb = (p.k0 + k - 1) * (long long)p.t.hop - p.t0;
     float* __restrict__ yr = p.x + row * p.x_row_stride;
     const bool accumulate = p.parity != 0;
@@ -293,6 +294,93 @@ __global__ void mirror_adj_kernel(const __grid_constant__ SlicqBinsParams p) {
         cv.x += v.x; cv.y += v.y;
         *c = cv;
     }
+}
+
+// ------------------------------------------------------------------------------------------
+// The long bin (SlicqLongBinParams: the Nyquist bin of a band-limited filterbank, too long for the bins kernels' register
+// codelets).  The formulas of the bins kernels (k_bins.cu), for one transform of length M per CTA on the Stockham engine
+// above, after bins_fwd_kernel / bins_inv_kernel on the same stream:
+//     analysis   c[n] = (-1)^n IDFT_M(H[hoff + m'] wf'[m'])[n]  -> the caller's bucket, and |c| (slicq_forward_norm);
+//                in the mask-gradient mode Re(conj(X) c) instead, X the mixture at row row % x_rows
+//     synthesis  T[off + m'] = wi'[m'] DFT_M((-1)^n c[n] (x mask[n], c from mixture row row % x_rows))[m'],
+//                off = ovoff for the leading ov coefficients, toff for the others; and the gap zero-fill of the bucket
+// Launch bound 3: the transform needs few registers, and short long bins (a few hundred coefficients) run 3 CTAs per SM.
+__global__ void __launch_bounds__(SLICQ_GEN_THREADS, 3) long_bin_fwd_kernel(const __grid_constant__ SlicqLongBinParams p) {
+    SLICQ_DYN_SMEM(float2, A);
+    const int M = p.M, NT = SLICQ_GEN_THREADS, tid = threadIdx.x;
+    float2* B = A + M;
+    const int u = blockIdx.x;
+    const int rs = p.rs0 + u;
+    const int row = rs / p.S, k = rs - row * p.S;
+    const float2* __restrict__ H = p.spec + (long long)u * p.spec_stride + p.hoff;
+    for (int m = tid; m < M; m += NT) {
+        const float2 h = H[m];
+        const float w = __ldg(p.w + m);
+        A[m] = make_float2(h.x * w, h.y * w);
+    }
+    __syncthreads();
+    const float2* Z = stockham<true>(A, B, M, p.n_fac, p.fac, p.wM, p.wP);
+    const SlicqBucketArg& b = p.b;
+    const int rowx = p.mask_grad ? row % p.x_rows : row;
+    float2* __restrict__ c = b.ptr + rowx * b.s_row + k * b.s_slice;
+    float* __restrict__ aux = b.nptr ? b.nptr + row * b.ms_row + k * b.ms_slice : nullptr;
+    for (int n = tid; n < M; n += NT) {
+        float2 v = Z[n];
+        if (n & 1) v = make_float2(-v.x, -v.y);
+        if (p.mask_grad) { aux[n] = mask_grad_of(c[n], v); continue; }
+        c[n] = v;
+        if (aux) aux[n] = sqrtf(fmaf(v.x, v.x, v.y * v.y));
+    }
+}
+
+__global__ void __launch_bounds__(SLICQ_GEN_THREADS, 3) long_bin_inv_kernel(const __grid_constant__ SlicqLongBinParams p) {
+    SLICQ_DYN_SMEM(float2, A);
+    const int M = p.M, NT = SLICQ_GEN_THREADS, tid = threadIdx.x;
+    float2* B = A + M;
+    const int u = blockIdx.x;
+    const int rs = p.rs0 + u;
+    const int row = rs / p.S, k = rs - row * p.S;
+    const SlicqBucketArg& b = p.b;
+    const float2* __restrict__ c = b.ptr + (p.x_rows ? row % p.x_rows : row) * b.s_row + k * b.s_slice;
+    const float* __restrict__ mk = b.mptr ? b.mptr + row * b.ms_row + k * b.ms_slice : nullptr;
+    for (int n = tid; n < M; n += NT) {
+        float2 v = c[n];
+        if (mk) { const float m = mk[n]; v.x *= m; v.y *= m; }
+        if (n & 1) v = make_float2(-v.x, -v.y);
+        A[n] = v;
+    }
+    __syncthreads();
+    const float2* Z = stockham<false>(A, B, M, p.n_fac, p.fac, p.wM, p.wP);
+    float2* __restrict__ T = p.spec + (long long)u * p.spec_stride;
+    for (int m = tid; m < M; m += NT) {
+        const float2 z = Z[m];
+        const float w = __ldg(p.w + m);
+        T[(m < p.ov ? p.ovoff : p.toff) + m] = make_float2(z.x * w, z.y * w);
+    }
+    // positions of the T planes that no bin covers and that this bucket owns (see SlicqDeviceTables)
+    for (int e = 0; e < p.gap_n; ++e) {
+        const int2 g = __ldg(p.gaps + e);
+        for (int i = tid; i < g.y; i += NT) T[g.x + i] = make_float2(0.f, 0.f);
+    }
+}
+
+extern "C" int slicq_long_bin_smem_bytes(int M) {
+    const long long b = 2LL * M * (long long)sizeof(float2);
+    return (M > 0 && b <= 220 * 1024) ? (int)b : -1;
+}
+
+extern "C" int slicq_launch_long_bin(const SlicqLongBinParams* p, int inverse, cudaStream_t s) {
+    if (p->n_rs <= 0) return 0;
+    const int smem = slicq_long_bin_smem_bytes(p->M);
+    if (smem < 0) return -2;
+    if (inverse) {
+        if (slicq_smem_opt_in<long_bin_inv_kernel>(smem)) return -3;
+        SLICQ_LAUNCH(long_bin_inv_kernel, dim3(p->n_rs), dim3(SLICQ_GEN_THREADS), smem, s, *p);
+    } else {
+        if (slicq_smem_opt_in<long_bin_fwd_kernel>(smem)) return -3;
+        SLICQ_LAUNCH(long_bin_fwd_kernel, dim3(p->n_rs), dim3(SLICQ_GEN_THREADS), smem, s, *p);
+    }
+    return (int)cudaGetLastError();
 }
 
 extern "C" int slicq_generic_smem_bytes(int L) {

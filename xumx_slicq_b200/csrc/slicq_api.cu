@@ -1,11 +1,14 @@
 // C-ABI of libslicq (include/slicq.h): plan construction and the chunked launch sequences.
 //
-// forward  : per chunk of (row,slice) units   slice_fft_fwd_kernel -> bins_fwd_kernel [-> mirror_adj_kernel]
-//            (slicq_forward_mask_grad: the same sequence, bins_fwd_kernel / mirror_adj_kernel in their mask-gradient mode)
-// inverse  : per chunk                         bins_inv_kernel [-> mirror_fix_kernel] -> slice_fft_inv_kernel (even slices,
-//                                              then odd slices)
+// forward  : per chunk of (row,slice) units   slice_fft_fwd_kernel -> bins_fwd_kernel [-> long_bin_fwd_kernel]
+//                                              [-> mirror_adj_kernel]
+//            (slicq_forward_mask_grad: the same sequence, the bins, long-bin and mirror_adj kernels in their mask-gradient
+//            mode)
+// inverse  : per chunk                         bins_inv_kernel [-> long_bin_inv_kernel] [-> mirror_fix_kernel] ->
+//                                              slice_fft_inv_kernel (even slices, then odd slices)
 //            (bins_inv_ovr_kernel in place of bins_inv_kernel for plans whose overflow spans several transform runs)
-// (the bracketed kernels only for bins that reach below DC; mirror_adj_kernel only in the adjoint-of-synthesis plan)
+// (the long-bin kernels only for a Nyquist bin longer than SLICQ_MAX_M (fmax below fs / 2); the mirror kernels only for
+// bins that reach below DC, mirror_adj_kernel only in the adjoint-of-synthesis plan)
 // A chunk's intermediate spectra (analysis: padded half spectra H; synthesis: the two bin planes T) live in the
 // caller-provided scratch buffer; SLICQ_CHUNK_MB bounds the chunk (default: one chunk per call).
 #include "slicq_common.cuh"
@@ -62,6 +65,8 @@ extern "C" int slicq_launch_slice_inv(const SlicqSliceParams* p, cudaStream_t s)
 extern "C" int slicq_slice_smem_bytes(int L);
 extern "C" int slicq_launch_mirror_fix(const SlicqBinsParams* p, cudaStream_t s);
 extern "C" int slicq_launch_mirror_adj(const SlicqBinsParams* p, cudaStream_t s);
+extern "C" int slicq_long_bin_smem_bytes(int M);
+extern "C" int slicq_launch_long_bin(const SlicqLongBinParams* p, int inverse, cudaStream_t s);
 
 namespace {
 
@@ -130,6 +135,7 @@ int fft_threads_per_transform(const FftPlan& f) {
 }
 
 struct Bucket {
+    bool is_long;    // the long bin (SlicqLongBinParams): no FftPlan, no jobs in the bins kernels
     int M, first_bin, n_bins, gt, tw_off, kind, A, B, smem_per_fft;
     int gap_first, gap_n;   // entries of the gap list (zero-filled positions of T) this bucket owns
     double cost;     // relative work per unit (for the job split)
@@ -154,6 +160,10 @@ struct slicq_plan {
     std::vector<void*> owned;
     int bins_smem;        // dynamic shared memory of the bins kernels
     bool ov_multi_run;    // a two-pass / prime bin diverts more than its first run of outputs: synthesis by bins_inv_ovr_kernel
+    bool has_long;        // the last bucket is the long bin: long_bin_*_kernel after each bins launch
+    SlicqLongBinParams lb;          // its tables (the per-launch fields are set by launch_long_bin)
+    const float* lb_wf;             // its analysis / synthesis windows in the device tables
+    const float* lb_wi;
     long long spec_stride_fwd;
     long long t_stride;   // complex elements per unit of the synthesis intermediate T
     long long chunk_bytes;
@@ -232,8 +242,14 @@ int check_bins(const slicq_tables& t, slicq_plan& p) {
     int off = 0;
     for (int j = 0; j < p.J; ++j) {
         const int M = p.bin_M[j], pos = p.bin_pos[j];
-        if (M < 4 || M % 4 != 0 || M > SLICQ_MAX_M || !find_fft_plan(M))
-            return fail(SLICQ_E_UNSUPPORTED, "bin length M must be a multiple of 4 in [16, 292]");
+        // the last (Nyquist) bin of a filterbank band-limited by fmax < fs / 2 may be longer: the long-bin kernels take it
+        const bool long_bin = j == p.J - 1 && M > SLICQ_MAX_M;
+        if (M < 4 || M % 4 != 0 || (!long_bin && !find_fft_plan(M)))
+            return fail(SLICQ_E_UNSUPPORTED, "bin length M must be a multiple of 4 in [16, 292]; only the last (Nyquist) "
+                                             "bin may be longer");
+        if (long_bin && slicq_long_bin_smem_bytes(M) < 0)
+            return fail(SLICQ_E_UNSUPPORTED, "the Nyquist bin does not fit the long-bin kernels' shared memory (two buffers "
+                                             "of M complex numbers)");
         // the lowest bins of Bark / mel filterbanks with few bins or a low fmin can share a position
         if (pos % 2 != 0 || pos < 0 || pos > p.N2 || (j > 0 && pos < p.bin_pos[j - 1]))
             return fail(SLICQ_E_UNSUPPORTED, "bin positions must be even, non-decreasing and within [0, L/2]");
@@ -250,16 +266,21 @@ int check_bins(const slicq_tables& t, slicq_plan& p) {
     return SLICQ_OK;
 }
 
-// buckets = maximal runs of equal M (nsgtf.py:66-78), their units per CTA iteration, shared memory, cost and twiddles
+// buckets = maximal runs of equal M (nsgtf.py:66-78), their units per CTA iteration, shared memory, cost and twiddles.  A
+// long last bin (M > SLICQ_MAX_M, see check_bins) is a bucket of its own, the last: its neighbour is at most SLICQ_MAX_M long
 int build_buckets(slicq_plan& p, PlanTables& h) {
     h.bin_bucket.resize(p.J);
     int tw_off = 0;
     for (int j = 0; j < p.J; ++j) {
         if (p.buckets.empty() || p.buckets.back().M != p.bin_M[j]) {
-            const FftPlan* f = find_fft_plan(p.bin_M[j]);
             Bucket b;
+            b.is_long = p.bin_M[j] > SLICQ_MAX_M;
             b.M = p.bin_M[j]; b.first_bin = j; b.n_bins = 0; b.tw_off = tw_off;
-            b.kind = f->kind; b.A = f->A; b.B = f->B; b.smem_per_fft = fft_smem_per_transform(*f);
+            b.kind = 0; b.A = 0; b.B = 0; b.smem_per_fft = 0;
+            if (!b.is_long) {
+                const FftPlan* f = find_fft_plan(p.bin_M[j]);
+                b.kind = f->kind; b.A = f->A; b.B = f->B; b.smem_per_fft = fft_smem_per_transform(*f);
+            }
             b.gt = 1; b.cost = 0.0; b.gap_first = 0; b.gap_n = 0;
             tw_off += b.M;
             p.buckets.push_back(b);
@@ -272,6 +293,7 @@ int build_buckets(slicq_plan& p, PlanTables& h) {
     // units per CTA iteration: fill the 256 threads of the hoisted pass, shared memory <= 48 KB
     p.bins_smem = 0;
     for (Bucket& b : p.buckets) {
+        if (b.is_long) continue;
         const FftPlan* f = find_fft_plan(b.M);
         int gt = kBinsThreads / (b.n_bins * fft_threads_per_transform(*f));
         if (gt < 1) gt = 1;
@@ -457,6 +479,25 @@ int build_mirror_entries(const slicq_tables& t, slicq_plan& p, PlanTables& h) {
     return SLICQ_OK;
 }
 
+// prime factors of n, largest first: the stages of the Stockham engine (k_slice_generic.cu)
+std::vector<int> prime_factors(int n) {
+    std::vector<int> fac;
+    for (int d = 2; d * d <= n; ++d) while (n % d == 0) { fac.push_back(d); n /= d; }
+    if (n > 1) fac.push_back(n);
+    std::sort(fac.begin(), fac.end(), [](int x, int y) { return x > y; });
+    return fac;
+}
+
+// the engine's double table for its first (largest) factor: exp(-2 pi i k / f) when f > 32, else one unused entry
+std::vector<double2> factor_twiddles(int f) {
+    std::vector<double2> w(f > 32 ? f : 1);
+    for (size_t kk = 0; kk < w.size(); ++kk) {
+        const double ang = -2.0 * M_PI * (double)kk / (double)w.size();
+        w[kk].x = cos(ang); w[kk].y = sin(ang);
+    }
+    return w;
+}
+
 // twiddles of the slice transforms: exp(-2 pi i k / L) of the real-FFT post-processing, and for the generic slice kernels
 // the prime factors of N2 (largest first) and exp(-2 pi i k / N2)
 int build_slice_tables(slicq_plan& p, PlanTables& h) {
@@ -466,17 +507,11 @@ int build_slice_tables(slicq_plan& p, PlanTables& h) {
         const double a = -2.0 * M_PI * (double)k / (double)p.L;
         h.post_tw[k] = make_float2((float)cos(a), (float)sin(a));
     }
-    std::vector<int> fac;
-    { int n = N2; for (int d = 2; d * d <= n; ++d) while (n % d == 0) { fac.push_back(d); n /= d; } if (n > 1) fac.push_back(n); }
-    std::sort(fac.begin(), fac.end(), [](int x, int y) { return x > y; });
+    const std::vector<int> fac = prime_factors(N2);
     if (fac.size() > 20) return fail(SLICQ_E_UNSUPPORTED, "too many prime factors in the slice length");
     p.dev.n_fac = (int)fac.size();
     for (size_t i = 0; i < fac.size(); ++i) p.dev.fac[i] = fac[i];
-    h.wP.resize(fac[0] > 32 ? fac[0] : 1);
-    for (size_t kk = 0; kk < h.wP.size(); ++kk) {
-        const double ang = -2.0 * M_PI * (double)kk / (double)h.wP.size();
-        h.wP[kk].x = cos(ang); h.wP[kk].y = sin(ang);
-    }
+    h.wP = factor_twiddles(fac[0]);
     h.wN.resize(N2);
     for (int kk = 0; kk < N2; ++kk) {
         const double ang = -2.0 * M_PI * (double)kk / (double)N2;
@@ -506,6 +541,29 @@ int upload_tables(slicq_plan& p, const PlanTables& h) {
     rc |= upload(h.wN, &d.wN, p.owned);
     rc |= upload(h.wP, &d.wP, p.owned);
     return rc ? fail(SLICQ_E_CUDA, "device table upload failed") : SLICQ_OK;
+}
+
+// the long bin's tables (SlicqLongBinParams), after the upload: its offsets, the prime factors of M and the double table of
+// the largest; exp(-2 pi i k / M), its windows and its gap list are its bucket's share of the device tables
+int build_long_bin(slicq_plan& p, const PlanTables& h) {
+    const Bucket& b = p.buckets.back();
+    p.has_long = b.is_long;
+    if (!p.has_long) return SLICQ_OK;
+    SlicqLongBinParams& l = p.lb;
+    memset(&l, 0, sizeof l);
+    const int j = b.first_bin;
+    l.M = b.M;
+    l.hoff = p.dev.pad_l + p.bin_pos[j] - b.M / 2;
+    l.toff = h.toff[j]; l.ov = h.ov[j]; l.ovoff = h.ovoff[j];
+    const std::vector<int> fac = prime_factors(b.M);
+    if (fac.size() > 20) return fail(SLICQ_E_UNSUPPORTED, "too many prime factors in the Nyquist bin's length");
+    l.n_fac = (int)fac.size();
+    for (size_t i = 0; i < fac.size(); ++i) l.fac[i] = fac[i];
+    l.wM = p.dev.tw + b.tw_off;
+    l.gaps = p.dev.gaps + b.gap_first; l.gap_n = b.gap_n;
+    p.lb_wf = p.dev.wf + p.bin_coff[j];
+    p.lb_wi = p.dev.wi + p.bin_coff[j];
+    return upload(factor_twiddles(fac[0]), &l.wP, p.owned) ? fail(SLICQ_E_CUDA, "device table upload failed") : SLICQ_OK;
 }
 
 }  // namespace
@@ -540,6 +598,7 @@ extern "C" int slicq_plan_create(const slicq_tables* t, slicq_plan** out) {
     if (int rc = build_mirror_entries(*t, *p, h)) return rc;
     if (int rc = build_slice_tables(*p, h)) return rc;
     if (int rc = upload_tables(*p, h)) return rc;
+    if (int rc = build_long_bin(*p, h)) return rc;
     p->spec_stride_fwd = (d.pad_l + p->N2 + 1 + d.pad_r + 1) & ~1LL;  // even: 16-byte aligned rows
     const char* env = getenv("SLICQ_CHUNK_MB");
     long long mb = env ? atoll(env) : 2048;
@@ -676,6 +735,10 @@ int fill_bins_params(const slicq_plan* p, const Call& c, SlicqBinsParams& bp, in
         a.mptr = c.aux && c.inverse ? reinterpret_cast<const float*>(c.aux[i].ptr) : nullptr;
         a.nptr = c.aux && !c.inverse ? reinterpret_cast<float*>(c.aux[i].ptr) : nullptr;
         a.ms_row = c.aux ? c.aux[i].s_row : 0; a.ms_bin = c.aux ? c.aux[i].s_bin : 0; a.ms_slice = c.aux ? c.aux[i].s_slice : 0;
+        if (b.is_long) {                                             // launch_long_bin's; the bins kernels see no job of it
+            a.units_per_job = n_rs; a.n_jobs = 0; a.job_start = jobs;
+            continue;
+        }
         const int groups = (n_rs + b.gt - 1) / b.gt;                 // iterations available in this chunk
         int nj = (int)(target * b.cost / total + 0.5);
         if (nj > groups) nj = groups;
@@ -687,6 +750,16 @@ int fill_bins_params(const slicq_plan* p, const Call& c, SlicqBinsParams& bp, in
         jobs += a.n_jobs;
     }
     return jobs;
+}
+
+// the long bin over the units of the bins launch `bp` (same chunk, views, row group and mode), right after it
+int launch_long_bin(const slicq_plan* p, const SlicqBinsParams& bp, bool inverse, cudaStream_t s) {
+    SlicqLongBinParams l = p->lb;
+    l.w = inverse ? p->lb_wi : p->lb_wf;
+    l.spec = bp.spec; l.spec_stride = bp.spec_stride;
+    l.n_rs = bp.n_rs; l.rs0 = bp.rs0; l.S = bp.S; l.x_rows = bp.x_rows; l.mask_grad = bp.mask_grad;
+    l.b = bp.b[bp.n_buckets - 1];
+    return slicq_launch_long_bin(&l, inverse ? 1 : 0, s);
 }
 
 int launch_result(int rc) {
@@ -710,7 +783,11 @@ int forward_one(const slicq_plan* p, const Call& c, void* scratch, cudaStream_t 
         ++g_launches;
         if (rc) break;
         const int jobs = fill_bins_params(p, c, *bp, n, (int)u0);
-        { ProfScope ps(K_BINS_FWD, s); rc = slicq_launch_bins(bp, jobs, p->bins_smem, bins_kernel(p, c), s); }
+        {
+            ProfScope ps(K_BINS_FWD, s);
+            rc = slicq_launch_bins(bp, jobs, p->bins_smem, bins_kernel(p, c), s);
+            if (!rc && p->has_long) { rc = launch_long_bin(p, *bp, false, s); ++g_launches; }
+        }
         ++g_launches;
         if (rc) break;
         if ((p->dev.adjoint & 1) && p->dev.n_mir > 0) {      // transpose of the mirrored-bin pass, reads this chunk's H
@@ -735,7 +812,11 @@ int inverse_one(const slicq_plan* p, const Call& c, void* scratch, cudaStream_t 
         // hops that the even slice has to have stored first (see slice_fft_inv_kernel)
         while (n > 1 && u0 + n < units && ((u0 + n) % c.n_slices) != 0 && (((u0 + n) % c.n_slices) & 1) == 0) --n;
         const int jobs = fill_bins_params(p, c, *bp, (int)n, (int)u0);
-        { ProfScope ps(K_BINS_INV, s); rc = slicq_launch_bins(bp, jobs, p->bins_smem, bins_kernel(p, c), s); }
+        {
+            ProfScope ps(K_BINS_INV, s);
+            rc = slicq_launch_bins(bp, jobs, p->bins_smem, bins_kernel(p, c), s);
+            if (!rc && p->has_long) { rc = launch_long_bin(p, *bp, true, s); ++g_launches; }
+        }
         ++g_launches;
         if (rc) break;
         if (p->dev.n_mir > 0) {          // mirrored-bin pass of configurations whose first bins reach below DC

@@ -321,6 +321,28 @@ struct SlicqSliceParams {
     int par_cs, par_base;  // ... one CTA each: par_cs = such slices per row, par_base = how many precede unit rs0 (set by the launcher)
 };
 
+// The long bin: the Nyquist bin of a filterbank band-limited by fmax < fs / 2 is as long as the band between fmax and fs / 2
+// (M > SLICQ_MAX_M).  It is the plan's last bucket, a bucket of one bin that the bins kernels skip; long_bin_fwd_kernel /
+// long_bin_inv_kernel (k_slice_generic.cu) transform it, one CTA per unit, in shared memory with the generic slice
+// kernels' Stockham engine, and do the gap zero-fill of its bucket.  The tables are the plan's; the rest is set per launch.
+struct SlicqLongBinParams {
+    int M;
+    int hoff;              // analysis: offset in a row of H of the bin's first coefficient (m' = 0): pad_l + pos - M / 2
+    int toff, ov, ovoff;   // synthesis: offset in a row of T of m' = 0, leading coefficients that go to the overflow slot,
+                           // offset of that slot
+    int n_fac;
+    int fac[20];           // prime factors of M, largest first
+    const float2* wM;      // [M] exp(-2 pi i k / M)
+    const double2* wP;     // exp(-2 pi i k / fac[0]) in double when fac[0] > 32
+    const float* w;        // [M] the bin's window in centred order: wf (analysis) or wi (synthesis)
+    const int2* gaps;      // synthesis: the T positions no bin writes that this bucket zero-fills ...
+    int gap_n;             // ... (entries)
+    float2* spec;          // as SlicqBinsParams
+    long long spec_stride;
+    int n_rs, rs0, S, x_rows, mask_grad;
+    SlicqBucketArg b;      // the caller's view of the bucket
+};
+
 // ---------------------------------------------------------------------------------------
 // host-side launcher helpers (k_bins.cu, k_slice.cu, k_slice_generic.cu)
 #include <atomic>
